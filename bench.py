@@ -3,12 +3,14 @@
 
     python bench.py --gpus N --steps K --warmup W              # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...     # CPU restatement of the reference (oracle port)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # + what the last timed step computed, as .npy
 
 Headline workload (BASELINE.json configs[1], "cfg2"): 128 scene graphs per GPU, 3-30 objects each (+ the
 __image__ dummy), VG-like vocabulary (50 predicates), WSGC canonicalization with learned converse +
 transitive edges, 5-layer GraphTripleConv stack (embed 128 / hidden 512) + box_net + box loss, the generator-side
 object embedding composited by boxes_to_layout into a 64x64x128 canvas on the GT boxes, backward through both, Adam.
-Synthetic graphs, random-init weights.  One JSON line on rank 0; see the prompt's bench contract for the keys.
+Synthetic graphs, random-init weights, all seeded: the same arguments give the same inputs in every run.  One JSON
+line on rank 0.
 
 The same line carries `configs`: BASELINE.json's other configurations measured in the same run
 (cfg1 CPU-sized step, cfg3 256x256 mask canvas, cfg4 CLEVR forward-only path, cfg5 ~1M-triple batch sharded over the
@@ -24,6 +26,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (no __pycache__)
 
 import numpy as np   # noqa: E402
 import torch         # noqa: E402
@@ -62,7 +65,15 @@ def parse():
     ap.add_argument("--profile", action="store_true",
                     help="profiling run: cudaProfilerStart/Stop around the timed region (ncu --profile-from-start off), "
                          "no e2e / CPU legs / extra configs; the printed numbers are not bench values")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy: its loss, its "
+                         "canonicalized triple count and every parameter after its Adam update (rank 0, ~23 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
+    return args
 
 
 def peaks():
@@ -336,6 +347,20 @@ def layout_roofline(boxes, off, max_objs, N, D, H, W, pk, masks=None, iters=20, 
             "bytes_per_launch": nbytes, "fwd": res["fwd"], "bwd": res["bwd"],
             "l2": "canvas of %.0f MB %s the 126 MB L2%s" % (nbytes / 1e6, "exceeds" if nbytes > 126e6 else "fits in",
                                                            "" if nbytes > 126e6 else "; L2 flushed between iterations")}
+
+
+def dump_outputs(out_dir, step, loss, n_tri):
+    """What the last timed step hands its caller, as <out_dir>/<name>.npy: the loss it returned, its canonicalized
+    triple count and every parameter after its Adam update (float32 / float64).  The inputs are seeded, so two builds
+    run with the same arguments can be compared file by file."""
+    step.finish()                  # under graph replay Adam of the last step runs on the look-ahead stream
+    arrays = {"loss": loss.detach().float().cpu().numpy(), "triples_after_canon": np.array(n_tri, np.float64)}
+    for prefix, module in (("model.", step.model), ("layout_embedding.", step.layout_embedding)):
+        for name, p in module.named_parameters():
+            arrays["param." + prefix + name] = p.detach().float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def mlp_flops(n_tri, n_obj, layers=5, train=True):
@@ -713,6 +738,8 @@ def run_ours(args):
         torch.cuda.cudart().cudaProfilerStop()
     launches = L.csg_launch_count() + step.graph_launches - launches0     # eager launch sites + those replayed from the graph
     sec = e0.elapsed_time(e1) * 1e-3
+    if args.dump_outputs and rank == 0:      # before the passes below train the same parameters further
+        dump_outputs(args.dump_outputs, step, loss, n_tri)
     # ---- instrumented pass (not the headline): the same K steps with CUDA events around every GEMM / layout /
     # pooling entry point on the launching stream (csg_prof_*), for the roofline objects
     import ctypes
