@@ -149,6 +149,40 @@ __device__ __forceinline__ unsigned short cvt16(float a, bool fp16) {
 // x > 0 for either format: sign bit clear and magnitude non-zero
 __device__ __forceinline__ bool pos16(uint32_t h) { return h != 0 && h < 0x8000u; }
 
+// ---- element access of the layout canvas and its gradient: float, __nv_bfloat16 or __half.  The 16-bit stores round
+// once to nearest even WITHOUT saturation (unlike pack2_16 / cvt16): the canvas is "the fp32 result, rounded", as
+// Tensor.to(dtype) rounds it -- fp16 overflow is +-inf and NaN stays NaN.  Loads widen exactly.
+__device__ __forceinline__ float to_f32(float x) { return x; }
+__device__ __forceinline__ float to_f32(__nv_bfloat16 x) { return __bfloat162float(x); }
+__device__ __forceinline__ float to_f32(__half x) { return __half2float(x); }
+template <typename T> __device__ __forceinline__ T from_f32(float x);
+template <> __device__ __forceinline__ float from_f32<float>(float x) { return x; }
+template <> __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float x) { return __float2bfloat16_rn(x); }
+template <> __device__ __forceinline__ __half from_f32<__half>(float x) { return __float2half_rn(x); }
+__device__ __forceinline__ uint32_t pack2_rn(float a, float b, __nv_bfloat16*) {
+  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+  return *reinterpret_cast<uint32_t*>(&h);
+}
+__device__ __forceinline__ uint32_t pack2_rn(float a, float b, __half*) {
+  __half2 h = __floats2half2_rn(a, b);
+  return *reinterpret_cast<uint32_t*>(&h);
+}
+// streaming store of 4 consecutive elements (16 B for fp32, 8 B for 16-bit; p aligned to that)
+__device__ __forceinline__ void st4_stream(float* p, float a, float b, float c, float d) { st_f4_stream(p, make_float4(a, b, c, d)); }
+template <typename T>
+__device__ __forceinline__ void st4_stream(T* p, float a, float b, float c, float d) {
+  __stcs(reinterpret_cast<uint2*>(p), make_uint2(pack2_rn(a, b, (T*)nullptr), pack2_rn(c, d, (T*)nullptr)));
+}
+// 8 consecutive elements widened to fp32 (32 B for fp32 = two 16-B loads, 16 B for 16-bit = one; p aligned to 16 B)
+__device__ __forceinline__ void ld8_f32(const float* p, float (&f)[8]) {
+  const float4 a = ld_f4(p), b = ld_f4(p + 4);
+  f[0] = a.x; f[1] = a.y; f[2] = a.z; f[3] = a.w; f[4] = b.x; f[5] = b.y; f[6] = b.z; f[7] = b.w;
+}
+__device__ __forceinline__ void ld8_f32(const __half* p, float (&f)[8]) { unpack8_16(*reinterpret_cast<const uint4*>(p), f, true); }
+__device__ __forceinline__ void ld8_f32(const __nv_bfloat16* p, float (&f)[8]) {
+  unpack8_16(*reinterpret_cast<const uint4*>(p), f, false);
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -33,6 +33,7 @@
 // with S = 8 for boxes_to_layout (layout.py:34) and S = M for masks_to_layout.
 #include "layout_common.cuh"
 #include <stdlib.h>
+#include <type_traits>
 
 // tensor-core backward (layout_bwd_tc.cu)
 bool csg_layout_bwd_tc_eligible(const float* dout, int N, int D, int H, int W, int max_objs);
@@ -40,6 +41,7 @@ size_t csg_layout_bwd_tc_partial_floats(int N, int NO, int D, int H, int W, int 
 int csg_layout_bwd_tc_launch(const float* dout, const float* masks, const int* obj_off, const float* axg, const float* ayg,
                              float* partial, float* dvecs, int N, int NO, int D, int H, int W, int M, int max_objs,
                              cudaStream_t stream);
+CSG_API size_t csg_layout_bwd_vecs_workspace(int N, int NO, int D, int H, int W);
 
 namespace {
 
@@ -170,8 +172,72 @@ __device__ void build_weights(const LayoutParams& p, const Smem& s, int L, int x
   __syncthreads();
 }
 
-template <bool HAS_MASK, int CH>
-__global__ void __launch_bounds__(NTHREADS) layout_fwd_kernel(LayoutParams p, float* __restrict__ out) {
+// acc[j][k] = sum over this warp's compacted objects, in list order, of vecs[o, d0 + j] * S_o(pixel k of this lane)
+template <bool HAS_MASK, int NC>
+__device__ __forceinline__ void accumulate(const LayoutParams& p, const Smem& s, const unsigned char* myact, int na,
+                                           int TW, int TH, int warp, int spx, int row, int col, int d0,
+                                           float (&acc)[NC][4]) {
+#pragma unroll
+  for (int j = 0; j < NC; ++j)
+#pragma unroll
+    for (int k = 0; k < 4; ++k) acc[j][k] = 0.f;
+  for (int a = 0; a < na; ++a) {
+    const int c = myact[a];
+    float4 w;
+    if (HAS_MASK) {
+      w = ld_f4(s.wS + c * TILE_PX + warp * STRIP_PX + spx);
+    } else {
+      const float wy = s.ay[c * TH + row];
+      w = ld_f4(s.ax + c * TW + col);
+      w.x *= wy; w.y *= wy; w.z *= wy; w.w *= wy;
+    }
+    const float* vp = s.vS + c * p.D + d0;
+#pragma unroll
+    for (int j4 = 0; j4 < NC; j4 += 4) {
+      const float4 v = ld_f4(vp + j4);
+      const float vv[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        acc[j4 + j][0] = fmaf(vv[j], w.x, acc[j4 + j][0]);
+        acc[j4 + j][1] = fmaf(vv[j], w.y, acc[j4 + j][1]);
+        acc[j4 + j][2] = fmaf(vv[j], w.z, acc[j4 + j][2]);
+        acc[j4 + j][3] = fmaf(vv[j], w.w, acc[j4 + j][3]);
+      }
+    }
+  }
+}
+
+// One pass over the tile's object list [*s_cursor, ...): list, weights, vectors and the per-warp compaction into
+// myact.  Returns the number of objects of this warp; *L / *more describe the list.
+template <bool HAS_MASK>
+__device__ __forceinline__ int build_pass(const LayoutParams& p, const Smem& s, int oend, int x0, int y0, int* s_cursor,
+                                          int* s_count, unsigned my_rows, unsigned char* myact, bool* more) {
+  const int tid = threadIdx.x, lane = tid & 31;
+  build_list(p, s.list, oend, x0, y0, s_cursor, s_count);
+  __syncthreads();
+  const int L = *s_count;
+  *more = *s_cursor < oend;   // read before the next build_list may advance it
+  build_weights<HAS_MASK>(p, s, L, x0, y0);
+  for (int i = tid; i < L * (p.D >> 2); i += NTHREADS) {
+    int c = i / (p.D >> 2), d4 = i % (p.D >> 2);
+    st_f4(s.vS + c * p.D + d4 * 4, ld_f4(p.vecs + (size_t)s.list[c] * p.D + d4 * 4));
+  }
+  // per-warp compaction: objects that touch this warp's strip (poisoned objects always do)
+  int na = 0;
+  for (int c0 = 0; c0 < L; c0 += 32) {
+    const int c = c0 + lane;
+    const bool keep = c < L && ((s.rowmask[c] & my_rows) != 0u || (s.flags[c] & 1));
+    const unsigned bal = __ballot_sync(0xffffffffu, keep);
+    if (keep) myact[na + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)c;
+    na += __popc(bal);
+  }
+  __syncthreads();
+  return na;
+}
+
+// T = float: the fp32 canvas.  T = __nv_bfloat16 / __half: the fp32 canvas rounded once to T (Tensor.to(T)).
+template <bool HAS_MASK, int CH, typename T>
+__global__ void __launch_bounds__(NTHREADS) layout_fwd_kernel(LayoutParams p, T* __restrict__ out) {
   CSG_PDL_WAIT();
   extern __shared__ __align__(16) float smem_raw[];
   __shared__ int s_cursor, s_count;
@@ -212,84 +278,138 @@ __global__ void __launch_bounds__(NTHREADS) layout_fwd_kernel(LayoutParams p, fl
   const bool active = y < p.H && x < p.W;
   const unsigned my_rows = ((1u << SR) - 1u) << (warp * SR);
   unsigned char* myact = s.act + warp * p.lcap;
-  bool first = true;
-  while (true) {
-    build_list(p, s.list, oend, x0, y0, &s_cursor, &s_count);
-    __syncthreads();
-    const int L = s_count;
-    const bool more = s_cursor < oend;   // read before the next build_list may advance it
-    build_weights<HAS_MASK>(p, s, L, x0, y0);
-    for (int i = tid; i < L * (p.D >> 2); i += NTHREADS) {
-      int c = i / (p.D >> 2), d4 = i % (p.D >> 2);
-      st_f4(s.vS + c * p.D + d4 * 4, ld_f4(p.vecs + (size_t)s.list[c] * p.D + d4 * 4));
-    }
-    // per-warp compaction: objects that touch this warp's strip (poisoned objects always do)
-    int na = 0;
-    for (int c0 = 0; c0 < L; c0 += 32) {
-      const int c = c0 + lane;
-      const bool keep = c < L && ((s.rowmask[c] & my_rows) != 0u || (s.flags[c] & 1));
-      const unsigned bal = __ballot_sync(0xffffffffu, keep);
-      if (keep) myact[na + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)c;
-      na += __popc(bal);
-    }
-    __syncthreads();
-    if (active) {
-      const size_t plane = (size_t)p.H * p.W;
-      float* dst = out + (size_t)n * p.D * plane + (size_t)y * p.W + x;      // channel 0 of this lane's pixels
-      for (int d0 = 0; d0 < p.D; d0 += CH) {
-        float acc[CH][4];
+  if constexpr (sizeof(T) == 4) {
+    // (the fp32 canvas keeps its own loop, written out, so that its code is exactly what it was before the 16-bit
+    // canvases were added)
+    bool first = true;
+    while (true) {
+      build_list(p, s.list, oend, x0, y0, &s_cursor, &s_count);
+      __syncthreads();
+      const int L = s_count;
+      const bool more = s_cursor < oend;   // read before the next build_list may advance it
+      build_weights<HAS_MASK>(p, s, L, x0, y0);
+      for (int i = tid; i < L * (p.D >> 2); i += NTHREADS) {
+        int c = i / (p.D >> 2), d4 = i % (p.D >> 2);
+        st_f4(s.vS + c * p.D + d4 * 4, ld_f4(p.vecs + (size_t)s.list[c] * p.D + d4 * 4));
+      }
+      // per-warp compaction: objects that touch this warp's strip (poisoned objects always do)
+      int na = 0;
+      for (int c0 = 0; c0 < L; c0 += 32) {
+        const int c = c0 + lane;
+        const bool keep = c < L && ((s.rowmask[c] & my_rows) != 0u || (s.flags[c] & 1));
+        const unsigned bal = __ballot_sync(0xffffffffu, keep);
+        if (keep) myact[na + __popc(bal & ((1u << lane) - 1u))] = (unsigned char)c;
+        na += __popc(bal);
+      }
+      __syncthreads();
+      if (active) {
+        const size_t plane = (size_t)p.H * p.W;
+        float* dst = out + (size_t)n * p.D * plane + (size_t)y * p.W + x;      // channel 0 of this lane's pixels
+        for (int d0 = 0; d0 < p.D; d0 += CH) {
+          float acc[CH][4];
 #pragma unroll
-        for (int j = 0; j < CH; ++j)
+          for (int j = 0; j < CH; ++j)
 #pragma unroll
-          for (int k = 0; k < 4; ++k) acc[j][k] = 0.f;
-        for (int a = 0; a < na; ++a) {
-          const int c = myact[a];
-          float4 w;
-          if (HAS_MASK) {
-            w = ld_f4(s.wS + c * TILE_PX + warp * STRIP_PX + spx);
-          } else {
-            const float wy = s.ay[c * TH + row];
-            w = ld_f4(s.ax + c * TW + col);
-            w.x *= wy; w.y *= wy; w.z *= wy; w.w *= wy;
-          }
-          const float* vp = s.vS + c * p.D + d0;
+            for (int k = 0; k < 4; ++k) acc[j][k] = 0.f;
+          for (int a = 0; a < na; ++a) {
+            const int c = myact[a];
+            float4 w;
+            if (HAS_MASK) {
+              w = ld_f4(s.wS + c * TILE_PX + warp * STRIP_PX + spx);
+            } else {
+              const float wy = s.ay[c * TH + row];
+              w = ld_f4(s.ax + c * TW + col);
+              w.x *= wy; w.y *= wy; w.z *= wy; w.w *= wy;
+            }
+            const float* vp = s.vS + c * p.D + d0;
 #pragma unroll
-          for (int j4 = 0; j4 < CH; j4 += 4) {
-            const float4 v = ld_f4(vp + j4);
-            const float vv[4] = {v.x, v.y, v.z, v.w};
+            for (int j4 = 0; j4 < CH; j4 += 4) {
+              const float4 v = ld_f4(vp + j4);
+              const float vv[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              acc[j4 + j][0] = fmaf(vv[j], w.x, acc[j4 + j][0]);
-              acc[j4 + j][1] = fmaf(vv[j], w.y, acc[j4 + j][1]);
-              acc[j4 + j][2] = fmaf(vv[j], w.z, acc[j4 + j][2]);
-              acc[j4 + j][3] = fmaf(vv[j], w.w, acc[j4 + j][3]);
+              for (int j = 0; j < 4; ++j) {
+                acc[j4 + j][0] = fmaf(vv[j], w.x, acc[j4 + j][0]);
+                acc[j4 + j][1] = fmaf(vv[j], w.y, acc[j4 + j][1]);
+                acc[j4 + j][2] = fmaf(vv[j], w.z, acc[j4 + j][2]);
+                acc[j4 + j][3] = fmaf(vv[j], w.w, acc[j4 + j][3]);
+              }
             }
           }
-        }
-        if (vec4 && first) {
-          // the common case: every canvas element is written exactly once, 16 bytes per lane, 512 contiguous
-          // bytes per warp and channel
+          if (vec4 && first) {
+            // the common case: every canvas element is written exactly once, 16 bytes per lane, 512 contiguous
+            // bytes per warp and channel
 #pragma unroll
-          for (int j = 0; j < CH; ++j, dst += plane)
-            st_f4_stream(dst, make_float4(acc[j][0], acc[j][1], acc[j][2], acc[j][3]));
-        } else {
+            for (int j = 0; j < CH; ++j, dst += plane)
+              st_f4_stream(dst, make_float4(acc[j][0], acc[j][1], acc[j][2], acc[j][3]));
+          } else {
 #pragma unroll
-          for (int j = 0; j < CH; ++j, dst += plane) {
-            if (vec4) {
-              float4 r = make_float4(acc[j][0], acc[j][1], acc[j][2], acc[j][3]);
-              float4 o = ld_f4(dst);
-              r.x += o.x; r.y += o.y; r.z += o.z; r.w += o.w;
-              st_f4_stream(dst, r);
-            } else {
-              for (int k = 0; k < 4 && x + k < p.W; ++k) dst[k] = first ? acc[j][k] : dst[k] + acc[j][k];
+            for (int j = 0; j < CH; ++j, dst += plane) {
+              if (vec4) {
+                float4 r = make_float4(acc[j][0], acc[j][1], acc[j][2], acc[j][3]);
+                float4 o = ld_f4(dst);
+                r.x += o.x; r.y += o.y; r.z += o.z; r.w += o.w;
+                st_f4_stream(dst, r);
+              } else {
+                for (int k = 0; k < 4 && x + k < p.W; ++k) dst[k] = first ? acc[j][k] : dst[k] + acc[j][k];
+              }
             }
           }
         }
       }
+      first = false;
+      __syncthreads();
+      if (!more) break;
     }
-    first = false;
-    __syncthreads();
-    if (!more) break;
+  } else {
+    // 16-bit canvas: every element is rounded once, from the same fp32 sum as the fp32 canvas.  A tile whose objects
+    // fit one list (the common case) is written as the fp32 kernel writes it, 8 bytes per lane, 256 contiguous bytes
+    // per warp and channel.  A tile that needs several passes keeps the running total tot = tot + acc_pass (the fp32
+    // canvas's out = out + acc) in registers for 4 channels at a time and rebuilds its lists for every channel group.
+    auto store = [&](T* dst, const float (&v)[4]) {
+      if (vec4) st4_stream(dst, v[0], v[1], v[2], v[3]);
+      else for (int k = 0; k < 4 && x + k < p.W; ++k) dst[k] = from_f32<T>(v[k]);
+    };
+    const size_t plane = (size_t)p.H * p.W;
+    T* dst0 = out + (size_t)n * p.D * plane + (size_t)y * p.W + x;
+    bool more;
+    int na = build_pass<HAS_MASK>(p, s, oend, x0, y0, &s_cursor, &s_count, my_rows, myact, &more);
+    if (!more) {
+      if (active) {
+        T* dst = dst0;
+        for (int d0 = 0; d0 < p.D; d0 += CH) {
+          float acc[CH][4];
+          accumulate<HAS_MASK, CH>(p, s, myact, na, TW, TH, warp, spx, row, col, d0, acc);
+#pragma unroll
+          for (int j = 0; j < CH; ++j, dst += plane) store(dst, acc[j]);
+        }
+      }
+      return;
+    }
+    constexpr int MC = 4;
+    for (int d0 = 0; d0 < p.D; d0 += MC) {
+      if (d0 > 0) {
+        __syncthreads();
+        if (tid == 0) s_cursor = p.obj_off[n];
+        __syncthreads();
+        na = build_pass<HAS_MASK>(p, s, oend, x0, y0, &s_cursor, &s_count, my_rows, myact, &more);
+      }
+      float tot[MC][4];
+      accumulate<HAS_MASK, MC>(p, s, myact, na, TW, TH, warp, spx, row, col, d0, tot);
+      while (more) {
+        __syncthreads();
+        na = build_pass<HAS_MASK>(p, s, oend, x0, y0, &s_cursor, &s_count, my_rows, myact, &more);
+        float acc[MC][4];
+        accumulate<HAS_MASK, MC>(p, s, myact, na, TW, TH, warp, spx, row, col, d0, acc);
+#pragma unroll
+        for (int j = 0; j < MC; ++j)
+#pragma unroll
+          for (int k = 0; k < 4; ++k) tot[j][k] = tot[j][k] + acc[j][k];
+      }
+      if (active) {
+#pragma unroll
+        for (int j = 0; j < MC; ++j) store(dst0 + (size_t)(d0 + j) * plane, tot[j]);
+      }
+    }
   }
 }
 
@@ -305,15 +425,22 @@ constexpr int BAND = 256;              // pixels per band (1 KB per channel)
 constexpr int SUBS = 8;                // consumer warps = 32-pixel sub-bands (8 + 1 warps per CTA, two CTAs per SM: the
                                        // per-object load -> FMA -> accumulate chains of one warp hide behind the others)
 constexpr int SUB_PX = BAND / SUBS;
-constexpr int CSTRIDE = BAND + 4;      // floats between channels of a stage: lanes (= channels) hit distinct banks
 constexpr int STAGES = 2;
-constexpr int STAGE_FLOATS = DC * CSTRIDE;
+// A stage holds DC channels x one band of the gradient in its own element type T (fp32: 1 KB, 16-bit: 512 B per channel,
+// one bulk copy each).  Channels are 16 B apart beyond the band, so that the 16-B loads of 8 consecutive lanes
+// (= channels) land on distinct bank groups: 260 floats for fp32, 264 halves for 16-bit.
+template <typename T>
+struct Stage {
+  static constexpr int CSTRIDE = BAND + 16 / (int)sizeof(T);        // elements between channels
+  static constexpr int FLOATS = DC * CSTRIDE * (int)sizeof(T) / 4;  // size of one stage in 4-byte words
+};
+constexpr int STAGE_FLOATS = Stage<float>::FLOATS;
 constexpr int NCONS = SUBS * 32;
 constexpr int NTHREADS = NCONS + 32;   // + producer warp
 
 struct Params {
   LayoutParams p;
-  const float* dout;
+  const void* dout;      // float, __nv_bfloat16 or __half (the kernel's T)
   float* partial;        // [splits][NO][D]
   const float* axg;      // [NO][W]  boxes: column factor; masks: column sample coordinate   (layout_tables_kernel)
   const float* ayg;      // [NO][H]
@@ -369,17 +496,17 @@ struct Smem {
   unsigned long long* bars;   // full[STAGES], empty[STAGES], tables
 };
 
-__host__ __device__ inline size_t smem_bytes(int lcap, int H, int W, bool mask) {
+__host__ __device__ inline size_t smem_bytes(int lcap, int H, int W, bool mask, int stage_floats = STAGE_FLOATS) {
   (void)H;   // the per-row factors stay in global memory (one L1-resident float per object visit)
-  size_t f = (size_t)STAGES * STAGE_FLOATS + (size_t)lcap * SUBS * DC + (size_t)lcap * W +
+  size_t f = (size_t)STAGES * stage_floats + (size_t)lcap * SUBS * DC + (size_t)lcap * W +
              (mask ? (size_t)lcap * BAND : 0) + (size_t)lcap * 4 + (size_t)lcap * SUBS / 4 /* act: SUBS * lcap bytes */;
   return f * 4 + (2 * STAGES + 1) * 8 + 16;
 }
 
-__device__ __forceinline__ Smem carve(float* base, int lcap, int H, int W, bool mask) {
+__device__ __forceinline__ Smem carve(float* base, int lcap, int H, int W, bool mask, int stage_floats) {
   Smem s;
   s.stage = base;
-  s.acc = s.stage + (size_t)STAGES * STAGE_FLOATS;
+  s.acc = s.stage + (size_t)STAGES * stage_floats;
   s.ax = s.acc + (size_t)lcap * SUBS * DC;
   s.wS = s.ax + (size_t)lcap * W;
   s.rng = reinterpret_cast<int*>(s.wS + (mask ? (size_t)lcap * BAND : 0));
@@ -428,12 +555,15 @@ __global__ void __launch_bounds__(128) layout_tables_kernel(LayoutParams p, int 
   if (threadIdx.x < 4) rng[4 * (size_t)o + threadIdx.x] = r[threadIdx.x];
 }
 
-template <bool HAS_MASK>
+// T: element type of the incoming gradient (float, __nv_bfloat16, __half); widened to fp32 as it leaves the stage, so the
+// sums are those of the fp32 kernel given the widened gradient.
+template <bool HAS_MASK, typename T>
 __global__ void __launch_bounds__(NTHREADS) layout_bwd_ring_kernel(Params q) {
   CSG_PDL_WAIT();
   extern __shared__ __align__(16) float smem_raw[];
+  constexpr int CSTRIDE = Stage<T>::CSTRIDE;
   const LayoutParams& p = q.p;
-  const Smem s = carve(smem_raw, p.lcap, p.H, p.W, HAS_MASK);
+  const Smem s = carve(smem_raw, p.lcap, p.H, p.W, HAS_MASK, Stage<T>::FLOATS);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int split = blockIdx.x % q.splits;
   const int cblk = (blockIdx.x / q.splits) % q.cblocks;
@@ -459,16 +589,16 @@ __global__ void __launch_bounds__(NTHREADS) layout_bwd_ring_kernel(Params q) {
 
   if (warp == SUBS) {
     // ---------------- producer: one 1 KB bulk copy per channel per band
-    const float* src0 = q.dout + ((size_t)n * p.D + cblk * DC + lane) * plane + (size_t)b0 * BAND;
+    const T* src0 = static_cast<const T*>(q.dout) + ((size_t)n * p.D + cblk * DC + lane) * plane + (size_t)b0 * BAND;
     int it = 0;
     for (int ch = 0; ch < nchunks; ++ch) {
       for (int b = 0; b < nb; ++b, ++it) {
         const int st = it % STAGES;
         if (it >= STAGES) mbar_wait(empty0 + 8 * st, ((it / STAGES) - 1) & 1);
-        if (lane == 0) mbar_arrive_expect_tx(full0 + 8 * st, DC * BAND * 4);
+        if (lane == 0) mbar_arrive_expect_tx(full0 + 8 * st, DC * BAND * sizeof(T));
         __syncwarp();
-        bulk_load(smem_u32(s.stage + (size_t)st * STAGE_FLOATS + lane * CSTRIDE), src0 + (size_t)b * BAND, BAND * 4,
-                  full0 + 8 * st);
+        bulk_load(smem_u32(reinterpret_cast<T*>(s.stage + (size_t)st * Stage<T>::FLOATS) + lane * CSTRIDE),
+                  src0 + (size_t)b * BAND, BAND * sizeof(T), full0 + 8 * st);
       }
     }
     return;
@@ -532,9 +662,19 @@ __global__ void __launch_bounds__(NTHREADS) layout_bwd_ring_kernel(Params q) {
       mbar_wait(full0 + 8 * st, (it / STAGES) & 1);
       float4 g[SUB_PX / 4];
       {
-        const float* gch = s.stage + (size_t)st * STAGE_FLOATS + lane * CSTRIDE + sub * SUB_PX;
+        const T* gch = reinterpret_cast<const T*>(s.stage + (size_t)st * Stage<T>::FLOATS) + lane * CSTRIDE + sub * SUB_PX;
+        if constexpr (sizeof(T) == 4) {
 #pragma unroll
-        for (int i = 0; i < SUB_PX / 4; ++i) g[i] = ld_f4(gch + 4 * i);
+          for (int i = 0; i < SUB_PX / 4; ++i) g[i] = ld_f4(gch + 4 * i);
+        } else {
+#pragma unroll
+          for (int i = 0; i < SUB_PX / 8; ++i) {
+            float f[8];
+            ld8_f32(gch + 8 * i, f);
+            g[2 * i] = make_float4(f[0], f[1], f[2], f[3]);
+            g[2 * i + 1] = make_float4(f[4], f[5], f[6], f[7]);
+          }
+        }
       }
       mbar_arrive(empty0 + 8 * st);          // the stage is free as soon as the registers hold it
       // Weights outside an object's column interval are exact zeros, so the dot product over the whole 32-pixel
@@ -620,15 +760,15 @@ struct Smem {
   unsigned* rowmask;   // [RR]      objects of the chunk whose factor changes behind row r
   unsigned long long* bars;
 };
-__host__ __device__ inline size_t smem_bytes(int lcap, int W, int RR) {
-  size_t f = (size_t)STAGES * STAGE_FLOATS + (size_t)lcap * SUBS * DC + (size_t)lcap * W + (size_t)lcap * RR +
+__host__ __device__ inline size_t smem_bytes(int lcap, int W, int RR, int stage_floats = STAGE_FLOATS) {
+  size_t f = (size_t)STAGES * stage_floats + (size_t)lcap * SUBS * DC + (size_t)lcap * W + (size_t)lcap * RR +
              (size_t)lcap * 4 + (size_t)RR;
   return f * 4 + (2 * STAGES + 1) * 8 + 16;
 }
-__device__ __forceinline__ Smem carve(float* base, int lcap, int W, int RR) {
+__device__ __forceinline__ Smem carve(float* base, int lcap, int W, int RR, int stage_floats) {
   Smem s;
   s.stage = base;
-  s.acc = s.stage + (size_t)STAGES * STAGE_FLOATS;
+  s.acc = s.stage + (size_t)STAGES * stage_floats;
   s.ax = s.acc + (size_t)lcap * SUBS * DC;
   s.day = s.ax + (size_t)lcap * W;
   s.rng = reinterpret_cast<int*>(s.day + (size_t)lcap * RR);
@@ -638,10 +778,12 @@ __device__ __forceinline__ Smem carve(float* base, int lcap, int W, int RR) {
   return s;
 }
 
-template <int SW>      // strip width: W = 8 * SW columns, one strip per consumer warp
+// SW: strip width, W = 8 * SW columns, one strip per consumer warp.  T: gradient element type, widened on load.
+template <int SW, typename T>
 __global__ void __launch_bounds__(NTHREADS) layout_bwd_colsum_kernel(Params q) {
   CSG_PDL_WAIT();
   extern __shared__ __align__(16) float smem_raw[];
+  constexpr int CSTRIDE = Stage<T>::CSTRIDE;
   constexpr int W = SW * SUBS;
   constexpr int RPB = BAND / W;          // rows per band
   static_assert(RPB * SW == SUB_PX, "a thread holds 32 gradient values per band");
@@ -654,7 +796,7 @@ __global__ void __launch_bounds__(NTHREADS) layout_bwd_colsum_kernel(Params q) {
   const int On = oend - obeg;
   const int b0 = split * q.bands_per_item, nb = q.bands_per_item;
   const int RR = nb * RPB, row0 = b0 * RPB;
-  const Smem s = carve(smem_raw, p.lcap, W, RR);
+  const Smem s = carve(smem_raw, p.lcap, W, RR, Stage<T>::FLOATS);
   const int nchunks = (On + p.lcap - 1) / p.lcap;
   const size_t plane = (size_t)p.H * W;
   float* my_partial = q.partial + ((size_t)split * q.NO + obeg) * p.D + cblk * DC;
@@ -672,16 +814,16 @@ __global__ void __launch_bounds__(NTHREADS) layout_bwd_colsum_kernel(Params q) {
 
   if (warp == SUBS) {
     // ---------------- producer: one 1 KB bulk copy per channel per band (as in the ring kernel)
-    const float* src0 = q.dout + ((size_t)n * p.D + cblk * DC + lane) * plane + (size_t)b0 * BAND;
+    const T* src0 = static_cast<const T*>(q.dout) + ((size_t)n * p.D + cblk * DC + lane) * plane + (size_t)b0 * BAND;
     int it = 0;
     for (int ch = 0; ch < nchunks; ++ch) {
       for (int b = 0; b < nb; ++b, ++it) {
         const int st = it % STAGES;
         if (it >= STAGES) mbar_wait(empty0 + 8 * st, ((it / STAGES) - 1) & 1);
-        if (lane == 0) mbar_arrive_expect_tx(full0 + 8 * st, DC * BAND * 4);
+        if (lane == 0) mbar_arrive_expect_tx(full0 + 8 * st, DC * BAND * sizeof(T));
         __syncwarp();
-        bulk_load(smem_u32(s.stage + (size_t)st * STAGE_FLOATS + lane * CSTRIDE), src0 + (size_t)b * BAND, BAND * 4,
-                  full0 + 8 * st);
+        bulk_load(smem_u32(reinterpret_cast<T*>(s.stage + (size_t)st * Stage<T>::FLOATS) + lane * CSTRIDE),
+                  src0 + (size_t)b * BAND, BAND * sizeof(T), full0 + 8 * st);
       }
     }
     return;
@@ -735,11 +877,23 @@ __global__ void __launch_bounds__(NTHREADS) layout_bwd_colsum_kernel(Params q) {
       mbar_wait(full0 + 8 * st, (it / STAGES) & 1);
       float4 g[SUB_PX / 4];
       {
-        const float* gch = s.stage + (size_t)st * STAGE_FLOATS + lane * CSTRIDE + sx0;
+        const T* gch = reinterpret_cast<const T*>(s.stage + (size_t)st * Stage<T>::FLOATS) + lane * CSTRIDE + sx0;
+        if constexpr (sizeof(T) == 4) {
 #pragma unroll
-        for (int k = 0; k < RPB; ++k)
+          for (int k = 0; k < RPB; ++k)
 #pragma unroll
-          for (int i = 0; i < SW / 4; ++i) g[k * (SW / 4) + i] = ld_f4(gch + k * W + 4 * i);
+            for (int i = 0; i < SW / 4; ++i) g[k * (SW / 4) + i] = ld_f4(gch + k * W + 4 * i);
+        } else {
+#pragma unroll
+          for (int k = 0; k < RPB; ++k)
+#pragma unroll
+            for (int i = 0; i < SW / 8; ++i) {
+              float f[8];
+              ld8_f32(gch + k * W + 8 * i, f);
+              g[k * (SW / 4) + 2 * i] = make_float4(f[0], f[1], f[2], f[3]);
+              g[k * (SW / 4) + 2 * i + 1] = make_float4(f[4], f[5], f[6], f[7]);
+            }
+        }
       }
       mbar_arrive(empty0 + 8 * st);          // the stage is free as soon as the registers hold it
 #pragma unroll
@@ -832,7 +986,7 @@ bool shape_ok(int D, int H, int W) {
 size_t workspace_bytes(int N, int NO, int D, int H, int W) {
   return ((size_t)pick_splits(N, D, H, W) * NO * D + (size_t)NO * (W + H) + (size_t)NO * 4) * 4 + 256;
 }
-bool eligible(const float* dout, int D, int H, int W) {
+bool eligible(const void* dout, int D, int H, int W) {
   return shape_ok(D, H, W) && (reinterpret_cast<uintptr_t>(dout) & 15) == 0;
 }
 
@@ -914,8 +1068,9 @@ __device__ void build_weights(const LayoutParams& p, const Smem& s, int L, int x
 
 constexpr int BWD_CH = 8;   // objects whose 8 weights per pixel slice are kept in registers
 
-template <bool HAS_MASK>
-__global__ void __launch_bounds__(NTHREADS) layout_bwd_vecs_kernel(LayoutParams p, const float* __restrict__ dout,
+// T: element type of the incoming gradient (float, __nv_bfloat16, __half), widened on load
+template <bool HAS_MASK, typename T>
+__global__ void __launch_bounds__(NTHREADS) layout_bwd_vecs_kernel(LayoutParams p, const T* __restrict__ dout,
                                                                   float* __restrict__ partial) {
   extern __shared__ __align__(16) float smem_raw[];
   __shared__ int s_cursor, s_count;
@@ -934,7 +1089,8 @@ __global__ void __launch_bounds__(NTHREADS) layout_bwd_vecs_kernel(LayoutParams 
   const int slice = tid & 63, cg = tid >> 6;       // 64 slices of 8 px, 4 channel groups
   const int row = slice >> 3, col8 = (slice & 7) * 8;
   const int y = y0 + row, x = x0 + col8;
-  const bool vec4 = (p.W & 3) == 0 && (reinterpret_cast<uintptr_t>(dout) & 15) == 0;
+  // 8 pixels per 16-B aligned load pair (fp32) or load (16-bit)
+  const bool vec4 = (p.W & (16 / (int)sizeof(T) - 1)) == 0 && (reinterpret_cast<uintptr_t>(dout) & 15) == 0;
   const bool rowok = y < p.H;
   while (true) {
     build_list(p, s.list, oend, x0, y0, &s_cursor, &s_count);
@@ -960,13 +1116,17 @@ __global__ void __launch_bounds__(NTHREADS) layout_bwd_vecs_kernel(LayoutParams 
       }
       for (int d = cg; d < p.D; d += 4) {
         float g[8];
-        const float* src = dout + (((size_t)n * p.D + d) * p.H + y) * p.W + x;
+        const T* src = dout + (((size_t)n * p.D + d) * p.H + y) * p.W + x;
         if (rowok && vec4 && x + 7 < p.W) {
-          float4 a = ld_f4_stream(src), b = ld_f4_stream(src + 4);
-          g[0] = a.x; g[1] = a.y; g[2] = a.z; g[3] = a.w; g[4] = b.x; g[5] = b.y; g[6] = b.z; g[7] = b.w;
+          if constexpr (sizeof(T) == 4) {
+            float4 a = ld_f4_stream(src), b = ld_f4_stream(src + 4);
+            g[0] = a.x; g[1] = a.y; g[2] = a.z; g[3] = a.w; g[4] = b.x; g[5] = b.y; g[6] = b.z; g[7] = b.w;
+          } else {
+            unpack8_16(__ldcs(reinterpret_cast<const uint4*>(src)), g, std::is_same<T, __half>::value);
+          }
         } else {
 #pragma unroll
-          for (int k = 0; k < 8; ++k) g[k] = (rowok && x + k < p.W) ? src[k] : 0.f;
+          for (int k = 0; k < 8; ++k) g[k] = (rowok && x + k < p.W) ? to_f32(src[k]) : 0.f;
         }
         float v[BWD_CH];
 #pragma unroll
@@ -1071,18 +1231,15 @@ int set_smem(K kernel, size_t smem) {
   return 0;
 }
 
-}  // namespace
-
-// ----------------------------------------------------------------------------------------
-// C ABI
-// ----------------------------------------------------------------------------------------
-CSG_API int csg_layout_fwd(const float* vecs, const float* boxes, const float* masks, const int* obj_off,
-                           const float* lin_x, const float* lin_y, float* out, int N, int D, int H, int W,
-                           int M, int align_corners, int max_objs_per_image, cudaStream_t stream) {
+// csg_layout_fwd with a canvas of element type T
+template <typename T>
+int layout_fwd(const float* vecs, const float* boxes, const float* masks, const int* obj_off, const float* lin_x,
+               const float* lin_y, T* out, int N, int D, int H, int W, int M, int align_corners, int max_objs_per_image,
+               cudaStream_t stream) {
   LayoutParams p;
   if (int rc = fill_params(p, vecs, boxes, masks, obj_off, lin_x, lin_y, N, D, H, W, M, align_corners)) return rc;
   if (N == 0) return 0;
-  CsgProfScope prof(CSG_PROF_LAYOUT_FWD, 4.0 * N * D * H * W, stream);
+  CsgProfScope prof(CSG_PROF_LAYOUT_FWD, (double)sizeof(T) * N * D * H * W, stream);
   p.TW = W <= 64 ? 64 : 128;
   p.TH = fw::TILE_PX / p.TW;
   p.tiles_x = csg_div_up(W, p.TW); p.tiles_y = csg_div_up(H, p.TH);
@@ -1101,8 +1258,8 @@ CSG_API int csg_layout_fwd(const float* vecs, const float* boxes, const float* m
   const bool wide = (D % 16) == 0;
 #define CSG_FWD_LAUNCH(MASK, CH)                                                          \
   do {                                                                                    \
-    if (int rc = set_smem(fw::layout_fwd_kernel<MASK, CH>, smem)) return rc;              \
-    CSG_CUDA(csg_launch_pdl(fw::layout_fwd_kernel<MASK, CH>, grid, dim3(fw::NTHREADS), smem, stream, p, out)); \
+    if (int rc = set_smem(fw::layout_fwd_kernel<MASK, CH, T>, smem)) return rc;           \
+    CSG_CUDA(csg_launch_pdl(fw::layout_fwd_kernel<MASK, CH, T>, grid, dim3(fw::NTHREADS), smem, stream, p, out)); \
   } while (0)
   if (masks) { if (wide) CSG_FWD_LAUNCH(true, 16); else CSG_FWD_LAUNCH(true, 4); }
   else       { if (wide) CSG_FWD_LAUNCH(false, 16); else CSG_FWD_LAUNCH(false, 4); }
@@ -1111,27 +1268,17 @@ CSG_API int csg_layout_fwd(const float* vecs, const float* boxes, const float* m
   return 0;
 }
 
-CSG_API size_t csg_layout_bwd_vecs_workspace(int N, int NO, int D, int H, int W) {
-  size_t need = gen::workspace_bytes(NO, D, H, W);
-  if (bw::shape_ok(D, H, W)) {
-    size_t ring = bw::workspace_bytes(N, NO, D, H, W);
-    if (ring > need) need = ring;
-  }
-  if (N > 0 && (D % 128) == 0 && (W % 32) == 0) {
-    size_t tc = (csg_layout_bwd_tc_partial_floats(N, NO, D, H, W, 16) + (size_t)NO * (W + H) + (size_t)NO * 4) * 4 + 256;
-    if (tc > need) need = tc;
-  }
-  return need;
-}
-
-CSG_API int csg_layout_bwd_vecs(const float* dout, const float* boxes, const float* masks, const int* obj_off,
-                                const float* lin_x, const float* lin_y, float* dvecs, int N, int NO, int D,
-                                int H, int W, int M, int align_corners, int max_objs_per_image,
-                                void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+// csg_layout_bwd_vecs with an incoming gradient of element type T.  The kernel, its schedule (bands, splits, rows per
+// CTA, object chunks) and its summation order are chosen from the shape alone, so a 16-bit gradient gives exactly the
+// dvecs of its fp32 widening.  The tcgen05 contraction (CSG_LAYOUT_BWD=tc) takes fp32 gradients only.
+template <typename T>
+int layout_bwd_vecs(const T* dout, const float* boxes, const float* masks, const int* obj_off, const float* lin_x,
+                    const float* lin_y, float* dvecs, int N, int NO, int D, int H, int W, int M, int align_corners,
+                    int max_objs_per_image, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   LayoutParams p;
   if (int rc = fill_params(p, nullptr, boxes, masks, obj_off, lin_x, lin_y, N, D, H, W, M, align_corners)) return rc;
   if (N == 0 || NO == 0) return 0;
-  CsgProfScope prof(CSG_PROF_LAYOUT_BWD, 4.0 * N * D * H * W, stream);
+  CsgProfScope prof(CSG_PROF_LAYOUT_BWD, (double)sizeof(T) * N * D * H * W, stream);
   CSG_REQUIRE(workspace_bytes >= csg_layout_bwd_vecs_workspace(N, NO, D, H, W), "layout bwd: workspace too small");
   float* partial = reinterpret_cast<float*>(workspace);
   // CSG_LAYOUT_BWD = tc | ring | generic forces a path (benchmarks).  Default: the ring kernel.  The tcgen05 3xTF32
@@ -1140,18 +1287,20 @@ CSG_API int csg_layout_bwd_vecs(const float* dout, const float* boxes, const flo
   // the 8 it needs per 32-pixel tile make it MMA-bound at 112 us on the cfg2 canvas (ring kernel: 81 us).
   static const char* force = getenv("CSG_LAYOUT_BWD");
   const bool want_tc = force && force[0] == 't';
-  if (want_tc && csg_layout_bwd_tc_eligible(dout, N, D, H, W, max_objs_per_image)) {
-    // tcgen05 path: dvecs = S * dout^T per image on the tensor cores (layout_bwd_tc.cu); tables as for the ring kernel
-    LayoutParams tp = p;
-    tp.TW = W; tp.TH = H; tp.tiles_x = tp.tiles_y = 1; tp.lcap = 0;
-    float* axg = partial + csg_layout_bwd_tc_partial_floats(N, NO, D, H, W, max_objs_per_image);
-    float* ayg = axg + (size_t)NO * W;
-    int* rng = reinterpret_cast<int*>(ayg + (size_t)NO * H);
-    if (masks) { CSG_CUDA(csg_launch_pdl(bw::layout_tables_kernel<true>, dim3(NO), dim3(128), 0, stream, tp, NO, axg, ayg, rng)); }
-    else       { CSG_CUDA(csg_launch_pdl(bw::layout_tables_kernel<false>, dim3(NO), dim3(128), 0, stream, tp, NO, axg, ayg, rng)); }
-    CSG_CHECK_LAUNCH("csg_layout_bwd_vecs tables");
-    return csg_layout_bwd_tc_launch(dout, masks, obj_off, axg, ayg, partial, dvecs, N, NO, D, H, W, M, max_objs_per_image,
-                                    stream);
+  if constexpr (sizeof(T) == 4) {
+    if (want_tc && csg_layout_bwd_tc_eligible(dout, N, D, H, W, max_objs_per_image)) {
+      // tcgen05 path: dvecs = S * dout^T per image on the tensor cores (layout_bwd_tc.cu); tables as for the ring kernel
+      LayoutParams tp = p;
+      tp.TW = W; tp.TH = H; tp.tiles_x = tp.tiles_y = 1; tp.lcap = 0;
+      float* axg = partial + csg_layout_bwd_tc_partial_floats(N, NO, D, H, W, max_objs_per_image);
+      float* ayg = axg + (size_t)NO * W;
+      int* rng = reinterpret_cast<int*>(ayg + (size_t)NO * H);
+      if (masks) { CSG_CUDA(csg_launch_pdl(bw::layout_tables_kernel<true>, dim3(NO), dim3(128), 0, stream, tp, NO, axg, ayg, rng)); }
+      else       { CSG_CUDA(csg_launch_pdl(bw::layout_tables_kernel<false>, dim3(NO), dim3(128), 0, stream, tp, NO, axg, ayg, rng)); }
+      CSG_CHECK_LAUNCH("csg_layout_bwd_vecs tables");
+      return csg_layout_bwd_tc_launch(dout, masks, obj_off, axg, ayg, partial, dvecs, N, NO, D, H, W, M, max_objs_per_image,
+                                      stream);
+    }
   }
   if ((!force || force[0] != 'g') && bw::eligible(dout, D, H, W)) {
     bw::Params q;
@@ -1175,11 +1324,11 @@ CSG_API int csg_layout_bwd_vecs(const float* dout, const float* boxes, const flo
     if (want_cs && RR <= bw::cs::RR_MAX) {
       // boxes: running column sums + summation by parts along y (layout_bwd_colsum_kernel)
       q.p.lcap = bw::cs::pick_lcap(max_objs_per_image, W, RR);
-      const size_t smem = bw::cs::smem_bytes(q.p.lcap, W, RR);
+      const size_t smem = bw::cs::smem_bytes(q.p.lcap, W, RR, bw::Stage<T>::FLOATS);
 #define CSG_CS_LAUNCH(SW)                                                                                       \
       do {                                                                                                      \
-        if (int rc = set_smem(bw::cs::layout_bwd_colsum_kernel<SW>, smem)) return rc;                           \
-        CSG_CUDA(csg_launch_pdl(bw::cs::layout_bwd_colsum_kernel<SW>, dim3(grid), dim3(bw::NTHREADS), smem, stream, q)); \
+        if (int rc = set_smem(bw::cs::layout_bwd_colsum_kernel<SW, T>, smem)) return rc;                        \
+        CSG_CUDA(csg_launch_pdl(bw::cs::layout_bwd_colsum_kernel<SW, T>, dim3(grid), dim3(bw::NTHREADS), smem, stream, q)); \
       } while (0)
       if (W == 64) CSG_CS_LAUNCH(8); else if (W == 128) CSG_CS_LAUNCH(16); else CSG_CS_LAUNCH(32);
 #undef CSG_CS_LAUNCH
@@ -1189,13 +1338,13 @@ CSG_API int csg_layout_bwd_vecs(const float* dout, const float* boxes, const flo
       CSG_CHECK_LAUNCH("csg_layout_bwd_vecs sum");
       return 0;
     }
-    const size_t smem = bw::smem_bytes(q.p.lcap, H, W, masks != nullptr);
+    const size_t smem = bw::smem_bytes(q.p.lcap, H, W, masks != nullptr, bw::Stage<T>::FLOATS);
     if (masks) {
-      if (int rc = set_smem(bw::layout_bwd_ring_kernel<true>, smem)) return rc;
-      CSG_CUDA(csg_launch_pdl(bw::layout_bwd_ring_kernel<true>, dim3(grid), dim3(bw::NTHREADS), smem, stream, q));
+      if (int rc = set_smem(bw::layout_bwd_ring_kernel<true, T>, smem)) return rc;
+      CSG_CUDA(csg_launch_pdl(bw::layout_bwd_ring_kernel<true, T>, dim3(grid), dim3(bw::NTHREADS), smem, stream, q));
     } else {
-      if (int rc = set_smem(bw::layout_bwd_ring_kernel<false>, smem)) return rc;
-      CSG_CUDA(csg_launch_pdl(bw::layout_bwd_ring_kernel<false>, dim3(grid), dim3(bw::NTHREADS), smem, stream, q));
+      if (int rc = set_smem(bw::layout_bwd_ring_kernel<false, T>, smem)) return rc;
+      CSG_CUDA(csg_launch_pdl(bw::layout_bwd_ring_kernel<false, T>, dim3(grid), dim3(bw::NTHREADS), smem, stream, q));
     }
     CSG_CHECK_LAUNCH("csg_layout_bwd_vecs ring");
     const long long n = (long long)NO * D;
@@ -1212,15 +1361,69 @@ CSG_API int csg_layout_bwd_vecs(const float* dout, const float* boxes, const flo
   dim3 grid(tiles, N);
   gen::obj_img_kernel<<<N, 64, 0, stream>>>(obj_off, N, obj_img);
   if (masks) {
-    if (int rc = set_smem(gen::layout_bwd_vecs_kernel<true>, smem)) return rc;
-    gen::layout_bwd_vecs_kernel<true><<<grid, gen::NTHREADS, smem, stream>>>(p, dout, partial);
+    if (int rc = set_smem(gen::layout_bwd_vecs_kernel<true, T>, smem)) return rc;
+    gen::layout_bwd_vecs_kernel<true, T><<<grid, gen::NTHREADS, smem, stream>>>(p, dout, partial);
   } else {
-    if (int rc = set_smem(gen::layout_bwd_vecs_kernel<false>, smem)) return rc;
-    gen::layout_bwd_vecs_kernel<false><<<grid, gen::NTHREADS, smem, stream>>>(p, dout, partial);
+    if (int rc = set_smem(gen::layout_bwd_vecs_kernel<false, T>, smem)) return rc;
+    gen::layout_bwd_vecs_kernel<false, T><<<grid, gen::NTHREADS, smem, stream>>>(p, dout, partial);
   }
   CSG_CHECK_LAUNCH("csg_layout_bwd_vecs");
   gen::layout_bwd_reduce_kernel<<<csg_div_up((long long)NO * D, 256), 256, 0, stream>>>(partial, obj_off, obj_img, dvecs,
                                                                                        NO, D, tiles);
   CSG_CHECK_LAUNCH("csg_layout_bwd_reduce");
   return 0;
+}
+
+}  // namespace
+
+// ----------------------------------------------------------------------------------------
+// C ABI
+// ----------------------------------------------------------------------------------------
+CSG_API int csg_layout_fwd(const float* vecs, const float* boxes, const float* masks, const int* obj_off,
+                           const float* lin_x, const float* lin_y, float* out, int N, int D, int H, int W,
+                           int M, int align_corners, int max_objs_per_image, cudaStream_t stream) {
+  return layout_fwd(vecs, boxes, masks, obj_off, lin_x, lin_y, out, N, D, H, W, M, align_corners, max_objs_per_image,
+                    stream);
+}
+
+CSG_API int csg_layout_fwd_bf16(const float* vecs, const float* boxes, const float* masks, const int* obj_off,
+                                const float* lin_x, const float* lin_y, void* out, int N, int D, int H, int W,
+                                int M, int align_corners, int max_objs_per_image, int fp16, cudaStream_t stream) {
+  if (fp16)
+    return layout_fwd(vecs, boxes, masks, obj_off, lin_x, lin_y, static_cast<__half*>(out), N, D, H, W, M,
+                      align_corners, max_objs_per_image, stream);
+  return layout_fwd(vecs, boxes, masks, obj_off, lin_x, lin_y, static_cast<__nv_bfloat16*>(out), N, D, H, W, M,
+                    align_corners, max_objs_per_image, stream);
+}
+
+CSG_API size_t csg_layout_bwd_vecs_workspace(int N, int NO, int D, int H, int W) {
+  size_t need = gen::workspace_bytes(NO, D, H, W);
+  if (bw::shape_ok(D, H, W)) {
+    size_t ring = bw::workspace_bytes(N, NO, D, H, W);
+    if (ring > need) need = ring;
+  }
+  if (N > 0 && (D % 128) == 0 && (W % 32) == 0) {
+    size_t tc = (csg_layout_bwd_tc_partial_floats(N, NO, D, H, W, 16) + (size_t)NO * (W + H) + (size_t)NO * 4) * 4 + 256;
+    if (tc > need) need = tc;
+  }
+  return need;
+}
+
+CSG_API int csg_layout_bwd_vecs(const float* dout, const float* boxes, const float* masks, const int* obj_off,
+                                const float* lin_x, const float* lin_y, float* dvecs, int N, int NO, int D,
+                                int H, int W, int M, int align_corners, int max_objs_per_image,
+                                void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  return layout_bwd_vecs(dout, boxes, masks, obj_off, lin_x, lin_y, dvecs, N, NO, D, H, W, M, align_corners,
+                         max_objs_per_image, workspace, workspace_bytes, stream);
+}
+
+CSG_API int csg_layout_bwd_vecs_bf16(const void* dout, const float* boxes, const float* masks, const int* obj_off,
+                                     const float* lin_x, const float* lin_y, float* dvecs, int N, int NO, int D,
+                                     int H, int W, int M, int align_corners, int max_objs_per_image, int fp16,
+                                     void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  if (fp16)
+    return layout_bwd_vecs(static_cast<const __half*>(dout), boxes, masks, obj_off, lin_x, lin_y, dvecs, N, NO, D, H, W,
+                           M, align_corners, max_objs_per_image, workspace, workspace_bytes, stream);
+  return layout_bwd_vecs(static_cast<const __nv_bfloat16*>(dout), boxes, masks, obj_off, lin_x, lin_y, dvecs, N, NO, D,
+                         H, W, M, align_corners, max_objs_per_image, workspace, workspace_bytes, stream);
 }

@@ -89,9 +89,11 @@ __global__ void __launch_bounds__(ORD_WARPS * 32) occlude_order_kernel(LayoutPar
 namespace occ {
 constexpr int TW = 64, TH = 8, NTHREADS = 128;
 
+// T: canvas element type (float, __nv_bfloat16, __half); a 16-bit canvas is the fp32 one rounded once
+template <typename T>
 __global__ void __launch_bounds__(NTHREADS) layout_occlude_kernel(LayoutParams p, const int* __restrict__ order,
                                                                   const int* __restrict__ img_flag,
-                                                                  float* __restrict__ out) {
+                                                                  T* __restrict__ out) {
   extern __shared__ __align__(16) float smem_raw[];
   __shared__ int s_cursor, s_count;
   float* cxs = smem_raw;                          // [lcap][TW] column sample coordinates
@@ -188,11 +190,11 @@ __global__ void __launch_bounds__(NTHREADS) layout_occlude_kernel(LayoutParams p
     }
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-      float* dst = out + (((size_t)n * p.D + d0 + j) * p.H + y) * p.W + x;
+      T* dst = out + (((size_t)n * p.D + d0 + j) * p.H + y) * p.W + x;
       if (vec4) {
-        st_f4_stream(dst, make_float4(v[0][j], v[1][j], v[2][j], v[3][j]));
+        st4_stream(dst, v[0][j], v[1][j], v[2][j], v[3][j]);
       } else {
-        for (int k = 0; k < 4 && x + k < p.W; ++k) dst[k] = v[k][j];
+        for (int k = 0; k < 4 && x + k < p.W; ++k) dst[k] = from_f32<T>(v[k][j]);
       }
     }
   }
@@ -214,9 +216,10 @@ namespace geom {
 constexpr int NTHREADS = 256;
 constexpr int RB = 8;      // canvas rows per pass
 
+template <typename T>
 struct Params {
   LayoutParams p;
-  const float* dout;
+  const T* dout;          // float, __nv_bfloat16 or __half: widened on load
   float* dboxes;    // [NO, 4]
   float* dmasks;    // [NO, M, M] or nullptr
   const int* obj_img;
@@ -255,8 +258,8 @@ __device__ __forceinline__ Smem carve(float* base, int D, int H, int W, int S) {
   return s;
 }
 
-template <bool HAS_MASK>
-__global__ void __launch_bounds__(NTHREADS) layout_bwd_geom_kernel(Params q) {
+template <bool HAS_MASK, typename T>
+__global__ void __launch_bounds__(NTHREADS) layout_bwd_geom_kernel(Params<T> q) {
   extern __shared__ __align__(16) float smem_raw[];
   const LayoutParams& p = q.p;
   const int S = HAS_MASK ? p.M : 8;
@@ -292,7 +295,7 @@ __global__ void __launch_bounds__(NTHREADS) layout_bwd_geom_kernel(Params q) {
   const int nx = xhi - xlo + 1;
   double ax0 = 0.0, axw = 0.0, ay0 = 0.0, ayh = 0.0;     // sums of g*dS/dix, g*dS/dix*u, g*dS/diy, g*dS/diy*v
   const size_t plane = (size_t)p.H * p.W;
-  const float* dimg = q.dout + (size_t)n * p.D * plane;
+  const T* dimg = q.dout + (size_t)n * p.D * plane;
 
   if (!poison && nx > 0) {
     for (int yb = ylo; yb <= yhi; yb += RB) {
@@ -300,9 +303,9 @@ __global__ void __launch_bounds__(NTHREADS) layout_bwd_geom_kernel(Params q) {
       // g[r][x] = sum_d dout[n, d, yb + r, x] * vec[d]
       for (int i = tid; i < nr * nx; i += NTHREADS) {
         const int r = i / nx, xx = xlo + i % nx;
-        const float* src = dimg + (size_t)(yb + r) * p.W + xx;
+        const T* src = dimg + (size_t)(yb + r) * p.W + xx;
         float acc = 0.f;
-        for (int d = 0; d < p.D; ++d) acc = fmaf(__ldg(src + (size_t)d * plane), s.vec[d], acc);
+        for (int d = 0; d < p.D; ++d) acc = fmaf(to_f32(__ldg(src + (size_t)d * plane)), s.vec[d], acc);
         s.g[r * p.W + xx] = acc;
       }
       __syncthreads();
@@ -404,10 +407,13 @@ CSG_API size_t csg_layout_occlude_workspace(int N, int NO) {
   return (size_t)NO * 8 + (size_t)NO * 4 + (size_t)(N + 1) * 4 + 64;
 }
 
-CSG_API int csg_layout_occlude_fwd(const float* vecs, const float* boxes, const float* masks, const int* obj_off,
-                                   const float* lin_x, const float* lin_y, float* out, int N, int NO, int D, int H,
-                                   int W, int M, int align_corners, void* workspace, size_t workspace_bytes,
-                                   cudaStream_t stream) {
+CSG_API size_t csg_layout_bwd_geom_workspace(int NO) { return (size_t)(NO + 1) * 4 + 64; }
+
+namespace {
+template <typename T>
+int layout_occlude_fwd(const float* vecs, const float* boxes, const float* masks, const int* obj_off, const float* lin_x,
+                       const float* lin_y, T* out, int N, int NO, int D, int H, int W, int M, int align_corners,
+                       void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   LayoutParams p;
   if (int rc = fill(p, vecs, boxes, masks, obj_off, lin_x, lin_y, N, D, H, W, M, align_corners)) return rc;
   CSG_REQUIRE(masks != nullptr, "layout occlude: masks are required (test_mode is a masks_to_layout feature)");
@@ -422,23 +428,21 @@ CSG_API int csg_layout_occlude_fwd(const float* vecs, const float* boxes, const 
   CSG_CHECK_LAUNCH("csg_layout_occlude_fwd order");
   p.lcap = 64;
   dim3 grid(p.tiles_x * p.tiles_y, N);
-  occ::layout_occlude_kernel<<<grid, occ::NTHREADS, occ::smem_bytes(p.lcap), stream>>>(p, order, flag, out);
+  occ::layout_occlude_kernel<T><<<grid, occ::NTHREADS, occ::smem_bytes(p.lcap), stream>>>(p, order, flag, out);
   CSG_CHECK_LAUNCH("csg_layout_occlude_fwd");
   return 0;
 }
 
-CSG_API size_t csg_layout_bwd_geom_workspace(int NO) { return (size_t)(NO + 1) * 4 + 64; }
-
-CSG_API int csg_layout_bwd_geom(const float* dout, const float* vecs, const float* boxes, const float* masks,
-                                const int* obj_off, const float* lin_x, const float* lin_y, float* dboxes,
-                                float* dmasks, int N, int NO, int D, int H, int W, int M, int align_corners,
-                                void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+template <typename T>
+int layout_bwd_geom(const T* dout, const float* vecs, const float* boxes, const float* masks, const int* obj_off,
+                    const float* lin_x, const float* lin_y, float* dboxes, float* dmasks, int N, int NO, int D, int H,
+                    int W, int M, int align_corners, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   LayoutParams p;
   if (int rc = fill(p, vecs, boxes, masks, obj_off, lin_x, lin_y, N, D, H, W, M, align_corners)) return rc;
   if (N == 0 || NO == 0) return 0;
   CSG_REQUIRE(workspace_bytes >= csg_layout_bwd_geom_workspace(NO), "layout bwd geom: workspace too small");
   CSG_REQUIRE(dboxes != nullptr, "layout bwd geom: dboxes is required");
-  geom::Params q;
+  geom::Params<T> q;
   q.p = p; q.dout = dout; q.dboxes = dboxes; q.dmasks = masks ? dmasks : nullptr; q.NO = NO;
   int* obj_img = reinterpret_cast<int*>(workspace);
   q.obj_img = obj_img;
@@ -448,12 +452,51 @@ CSG_API int csg_layout_bwd_geom(const float* dout, const float* vecs, const floa
   const size_t smem = geom::smem_bytes(D, H, W, S);
   CSG_REQUIRE(smem <= 220 * 1024, "layout bwd geom: D=%d H=%d W=%d M=%d need %zu bytes of shared memory", D, H, W, M, smem);
   if (masks) {
-    CSG_CUDA(cudaFuncSetAttribute(geom::layout_bwd_geom_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    geom::layout_bwd_geom_kernel<true><<<NO, geom::NTHREADS, smem, stream>>>(q);
+    CSG_CUDA(cudaFuncSetAttribute(geom::layout_bwd_geom_kernel<true, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    geom::layout_bwd_geom_kernel<true, T><<<NO, geom::NTHREADS, smem, stream>>>(q);
   } else {
-    CSG_CUDA(cudaFuncSetAttribute(geom::layout_bwd_geom_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    geom::layout_bwd_geom_kernel<false><<<NO, geom::NTHREADS, smem, stream>>>(q);
+    CSG_CUDA(cudaFuncSetAttribute(geom::layout_bwd_geom_kernel<false, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    geom::layout_bwd_geom_kernel<false, T><<<NO, geom::NTHREADS, smem, stream>>>(q);
   }
   CSG_CHECK_LAUNCH("csg_layout_bwd_geom");
   return 0;
+}
+}  // namespace
+
+CSG_API int csg_layout_occlude_fwd(const float* vecs, const float* boxes, const float* masks, const int* obj_off,
+                                   const float* lin_x, const float* lin_y, float* out, int N, int NO, int D, int H,
+                                   int W, int M, int align_corners, void* workspace, size_t workspace_bytes,
+                                   cudaStream_t stream) {
+  return layout_occlude_fwd(vecs, boxes, masks, obj_off, lin_x, lin_y, out, N, NO, D, H, W, M, align_corners, workspace,
+                            workspace_bytes, stream);
+}
+
+CSG_API int csg_layout_occlude_fwd_bf16(const float* vecs, const float* boxes, const float* masks, const int* obj_off,
+                                        const float* lin_x, const float* lin_y, void* out, int N, int NO, int D, int H,
+                                        int W, int M, int align_corners, int fp16, void* workspace,
+                                        size_t workspace_bytes, cudaStream_t stream) {
+  if (fp16)
+    return layout_occlude_fwd(vecs, boxes, masks, obj_off, lin_x, lin_y, static_cast<__half*>(out), N, NO, D, H, W, M,
+                              align_corners, workspace, workspace_bytes, stream);
+  return layout_occlude_fwd(vecs, boxes, masks, obj_off, lin_x, lin_y, static_cast<__nv_bfloat16*>(out), N, NO, D, H, W,
+                            M, align_corners, workspace, workspace_bytes, stream);
+}
+
+CSG_API int csg_layout_bwd_geom(const float* dout, const float* vecs, const float* boxes, const float* masks,
+                                const int* obj_off, const float* lin_x, const float* lin_y, float* dboxes,
+                                float* dmasks, int N, int NO, int D, int H, int W, int M, int align_corners,
+                                void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  return layout_bwd_geom(dout, vecs, boxes, masks, obj_off, lin_x, lin_y, dboxes, dmasks, N, NO, D, H, W, M,
+                         align_corners, workspace, workspace_bytes, stream);
+}
+
+CSG_API int csg_layout_bwd_geom_bf16(const void* dout, const float* vecs, const float* boxes, const float* masks,
+                                     const int* obj_off, const float* lin_x, const float* lin_y, float* dboxes,
+                                     float* dmasks, int N, int NO, int D, int H, int W, int M, int align_corners,
+                                     int fp16, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  if (fp16)
+    return layout_bwd_geom(static_cast<const __half*>(dout), vecs, boxes, masks, obj_off, lin_x, lin_y, dboxes, dmasks,
+                           N, NO, D, H, W, M, align_corners, workspace, workspace_bytes, stream);
+  return layout_bwd_geom(static_cast<const __nv_bfloat16*>(dout), vecs, boxes, masks, obj_off, lin_x, lin_y, dboxes,
+                         dmasks, N, NO, D, H, W, M, align_corners, workspace, workspace_bytes, stream);
 }

@@ -94,12 +94,18 @@ class HostBatch:
 class SgToLayoutStep:
     def __init__(self, vocab, device, precision="fp32", H=64, W=64, learned_converse=True,
                  learned_transitivity=True, lr=1e-4, seed=0, distributed=False, bbox_pred_loss_weight=10.0,
-                 global_batch=None, use_graph=False):
+                 global_batch=None, use_graph=False, canvas_dtype=torch.float32):
         """``global_batch``: number of graphs of the GLOBAL batch this rank holds a shard of.  The box loss is a mean
         over images (pix2pix_model.py:85), so with shards of unequal graph counts (cost-balanced sharding) every rank
         scales its loss by B_local / B_global and the gradients are SUMMED over ranks: the result equals the
         single-GPU gradient of the concatenated batch.  ``None``: every rank has the same number of graphs and the
-        gradients are averaged (the reference's DataParallel behaviour, meta_models.py:17)."""
+        gradients are averaged (the reference's DataParallel behaviour, meta_models.py:17).
+
+        ``canvas_dtype``: element type of the canvas and of the ``canvas_grad`` that ``step`` takes (``torch.float32``,
+        ``torch.bfloat16`` or ``torch.float16``), e.g. the dtype a mixed-precision generator consumes it in."""
+        if canvas_dtype not in (torch.float32, torch.bfloat16, torch.float16):
+            raise ValueError("canvas_dtype must be torch.float32, torch.bfloat16 or torch.float16")
+        self.canvas_dtype = canvas_dtype
         self.vocab, self.device, self.H, self.W = vocab, device, H, W
         self.flags = (learned_converse, learned_transitivity)
         self.model = Sg2LayoutModel(build_opt(vocab), precision=precision).to(device)
@@ -204,7 +210,7 @@ class SgToLayoutStep:
         with torch.cuda.stream(branch):
             layout_vecs = self.layout_embedding(d["objs"])
             canvas = layout_batched(layout_vecs, d["boxes"], d["obj_off"], self.H, self.W,
-                                    max_objs_per_image=d["max_objs"])
+                                    max_objs_per_image=d["max_objs"], out_dtype=self.canvas_dtype)
         obj_vecs, boxes_pred = self.model.forward_ragged(d["objs"], res.triplets, res.triplet_type, res.tri_off,
                                                          d["obj_off"])
         if branch is not main:
@@ -325,6 +331,8 @@ class SgToLayoutStep:
     def step(self, d, canvas_grad, prefetch=None):
         """One training step on batch ``d``.  ``prefetch``: the batch of the NEXT step (may be ``d`` itself); its
         canonicalization counting pass is enqueued right behind this step's emit pass."""
+        if canvas_grad.dtype != self.canvas_dtype:
+            raise ValueError("canvas_grad is %s, the canvas is %s" % (canvas_grad.dtype, self.canvas_dtype))
         if d.get("_ready") is not None:            # `d` was uploaded on the look-ahead stream
             torch.cuda.current_stream().wait_event(d["_ready"])
         if self.use_graph:
@@ -366,11 +374,15 @@ class SgToLayoutInference:
         (generator.py:16,80)  ->  masks_to_layout(test_mode=True) occlusion compositor on the PREDICTED boxes
         (layout.py:48-77,135-147), dummy objects removed (utils.py:56-63)
 
-    ``step(d)`` expects the device tensors of :class:`HostBatch` plus ``centers [NO, 2]`` and ``masks [NO, M, M]``."""
+    ``step(d)`` expects the device tensors of :class:`HostBatch` plus ``centers [NO, 2]`` and ``masks [NO, M, M]``;
+    the canvas it returns has dtype ``canvas_dtype`` (fp32, or the fp32 canvas rounded once to bf16 / fp16)."""
 
     def __init__(self, vocab, device, precision="fp16", H=256, W=256, embedding_dim=32, attr_sizes=None,
-                 learned_converse=True, learned_transitivity=True, seed=0):
+                 learned_converse=True, learned_transitivity=True, seed=0, canvas_dtype=torch.float32):
         import argparse
+        if canvas_dtype not in (torch.float32, torch.bfloat16, torch.float16):
+            raise ValueError("canvas_dtype must be torch.float32, torch.bfloat16 or torch.float16")
+        self.canvas_dtype = canvas_dtype
         self.vocab, self.device, self.H, self.W = vocab, device, H, W
         self.flags = (learned_converse, learned_transitivity)
         A = vocab.num_attributes
@@ -417,5 +429,5 @@ class SgToLayoutInference:
         dummy = (d["objs"][:, :1] == 0)
         boxes = torch.where(dummy, torch.full_like(boxes_pred, -1.0), boxes_pred.float())
         canvas = layout_batched(self.layout_embedding(d["objs"]), boxes, d["obj_off"], self.H, self.W, masks=d["masks"],
-                                test_mode=True)
+                                test_mode=True, out_dtype=self.canvas_dtype)
         return canvas, boxes_pred, int(res.triplets.shape[0])

@@ -80,6 +80,25 @@ int csg_layout_bwd_geom(const float* dout, const float* vecs, const float* boxes
                         const int* obj_off, const float* lin_x, const float* lin_y, float* dboxes,
                         float* dmasks, int N, int NO, int D, int H, int W, int M, int align_corners,
                         void* workspace, size_t workspace_bytes, csg_stream_t stream);
+/* 16-bit canvases (fp16 = 0: bf16, 1: fp16).  Forward: `out` is the fp32 canvas of the entry point above rounded once
+ * to nearest even (Tensor.to: fp16 overflow is +-inf, NaN stays NaN).  Backward: `dout` is widened on load; dvecs,
+ * dboxes and dmasks are bitwise those of the fp32 entry points given the widened gradient.  vecs, boxes, masks and
+ * all gradients stay fp32; the workspace queries above apply unchanged. */
+int csg_layout_fwd_bf16(const float* vecs, const float* boxes, const float* masks, const int* obj_off,
+                        const float* lin_x, const float* lin_y, void* out, int N, int D, int H, int W,
+                        int M, int align_corners, int max_objs_per_image, int fp16, csg_stream_t stream);
+int csg_layout_bwd_vecs_bf16(const void* dout, const float* boxes, const float* masks, const int* obj_off,
+                             const float* lin_x, const float* lin_y, float* dvecs, int N, int NO, int D,
+                             int H, int W, int M, int align_corners, int max_objs_per_image, int fp16,
+                             void* workspace, size_t workspace_bytes, csg_stream_t stream);
+int csg_layout_occlude_fwd_bf16(const float* vecs, const float* boxes, const float* masks, const int* obj_off,
+                                const float* lin_x, const float* lin_y, void* out, int N, int NO, int D, int H,
+                                int W, int M, int align_corners, int fp16, void* workspace, size_t workspace_bytes,
+                                csg_stream_t stream);
+int csg_layout_bwd_geom_bf16(const void* dout, const float* vecs, const float* boxes, const float* masks,
+                             const int* obj_off, const float* lin_x, const float* lin_y, float* dboxes,
+                             float* dmasks, int N, int NO, int D, int H, int W, int M, int align_corners,
+                             int fp16, void* workspace, size_t workspace_bytes, csg_stream_t stream);
 
 /* ---- box crops: sg2im/bilinear.py:65-94 (crop_bbox, backend 'cudnn'), :44-62 (crop_bbox_batch_cudnn).
  *      Crops crop_off[n]..crop_off[n+1] sample image n of feats [N,C,H,W] in place (the reference expands the
