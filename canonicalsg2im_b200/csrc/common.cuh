@@ -183,6 +183,21 @@ __device__ __forceinline__ void ld8_f32(const __nv_bfloat16* p, float (&f)[8]) {
   unpack8_16(*reinterpret_cast<const uint4*>(p), f, false);
 }
 
+// Calls f with a null pointer of the element type selected by fmt (0 fp32, 1 bf16, 2 fp16 -- the format codes of the
+// entry points that take any of the three), so one launch site covers every format; any other code is an error.
+#include <type_traits>
+template <typename F>
+static inline int csg_with_format(int fmt, F&& f) {
+  switch (fmt) {
+    case 0: return f((float*)nullptr);
+    case 1: return f((__nv_bfloat16*)nullptr);
+    case 2: return f((__half*)nullptr);
+  }
+  csg_set_error("element format %d is not 0 (fp32), 1 (bf16) or 2 (fp16)", fmt);
+  return 1;
+}
+template <typename P> using csg_elem_t = std::remove_pointer_t<P>;
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

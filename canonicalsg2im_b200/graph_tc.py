@@ -135,6 +135,8 @@ def invalidate_weight_copies(params=None):
     for e in _WCOPIES.values():
         if ptrs is None or ptrs & {q.data_ptr() for q in e["params"]}:
             e["versions"] = None
+    from . import mask_head       # the mask head's 3x3 convolution weights are cached on the same terms
+    mask_head.invalidate_weight_copies(params)
 
 
 def refresh_weight_copies(layers, act=BF):

@@ -4,8 +4,10 @@
 State-dict keys equal the reference's (``attribute_embedding.att_emb_{k}.weight``,
 ``pred_embeddings.weight``, ``trans_candidates_weights``, ``converse_candidates_weights``,
 ``gconvs.{i}.net1.{0,2}.*``, ``gconvs.{i}.net2.{0,2}.*``, ``gconvs.{i}.predicates_transitive_weights``,
-``box_net.{0,2}.*``), so reference checkpoints load with ``strict=True`` when ``mask_size == 0``.
-The optional cuDNN ``mask_net`` conv stack (``model.py:62-75``) is outside the hot path and not built.
+``box_net.{0,2}.*``, and with ``mask_size > 0`` the mask head's ``mask_net.{1,5,9,..}.*`` BatchNorm2d,
+``mask_net.{2,6,10,..}.*`` Conv2d and ``mask_net.{4k}.*`` 1x1 Conv2d), so reference checkpoints load with ``strict=True``.
+The mask head (``model.py:62-75``) runs on the csg2im kernels too (``mask_head.py``): its convolutions are GEMMs on the
+same engines as the GCN, with BatchNorm, upsampling and the patch gathers as memory-bound kernels around them.
 """
 import os
 
@@ -211,8 +213,6 @@ class Sg2LayoutModel(nn.Module):
         init = args.get("learned_init", "uniform")
         self.trans_candidates_weights = get_predicates_weights(num_preds, init)
         self.converse_candidates_weights = get_predicates_weights((num_preds, num_preds), init)
-        if (args.get("mask_size") or 0) > 0:
-            raise NotImplementedError("mask_net (cuDNN conv stack, model.py:62-75) is outside the csg2im hot path")
         gdim, hdim = args["gconv_dim"], args["gconv_hidden_dim"]
         self.gconvs = nn.ModuleList()
         d_obj, d_pred = num_attributes * emb, emb
@@ -225,6 +225,10 @@ class Sg2LayoutModel(nn.Module):
             d_obj, d_pred = gdim, gdim
         self.box_net = build_mlp([gdim, hdim, 4], final_nonlinearity=None)      # model.py:58-60
         self.mask_net = None
+        mask_size = args.get("mask_size") or 0
+        if mask_size > 0:
+            from .mask_head import build_mask_net
+            self.mask_net = build_mask_net(gdim, mask_size)       # model.py:62-75
         self.padding_id = self.vocab["pred_name_to_idx"]["__padding__"]
 
     def _act_dtype(self):
@@ -259,6 +263,9 @@ class Sg2LayoutModel(nn.Module):
         if self.precision in ("bf16", "fp16"):
             from . import graph_tc
             graph_tc.refresh_weight_copies(list(self.gconvs), self._act_dtype())
+            if self.mask_net is not None:
+                from . import mask_head
+                mask_head.refresh_weight_copies(self.mask_net, self._act_dtype())
 
     def _run(self, batch, obj_vecs, pred_vecs, first=0):
         layers = list(self.gconvs)[first:]
@@ -276,13 +283,27 @@ class Sg2LayoutModel(nn.Module):
                            self.box_net[2].weight, self.box_net[2].bias, False, self.precision)
         return obj_vecs, boxes
 
+    def masks_from_vecs(self, obj_vecs):
+        """The mask head (model.py:62-75,121-123) on object vectors [NO, D] (the GCN's output) -> masks_pred [NO, M, M]
+        fp32 in (0, 1).  BatchNorm uses the batch statistics of exactly these rows in training mode (and updates the
+        running buffers), the running buffers in eval mode.  Needs ``mask_size > 0``."""
+        if self.mask_net is None:
+            raise ValueError("masks_from_vecs needs a model built with mask_size > 0")
+        from .mask_head import mask_head
+        return mask_head(self.mask_net, obj_vecs, self.precision)
+
     def forward(self, objs, triplets, triplet_type, boxes_gt=None, masks_gt=None):
         """Padded interface (model.py:90-124): objs [B,O,A] i64, triplets [B,T,3] i64, triplet_type [B,T] i64
-        -> (obj_vecs [B,O,D], boxes_pred [B,O,4], None)."""
+        -> (obj_vecs [B,O,D], boxes_pred [B,O,4], masks_pred [B,O,M,M] or None when mask_size == 0).  The mask head
+        sees every row of the padded batch, padded objects included, as the box head does."""
         B, O, T = objs.size(0), objs.size(1), triplets.size(1)
         batch = TripleBatch.from_padded_triplets(triplets, triplet_type, self.padding_id, O, self.num_preds)
         obj_vecs, boxes = self._embed_and_run(batch, objs.reshape(B * O, -1), triplets.reshape(B * T, 3)[:, 1])
-        return obj_vecs.view(B, O, -1), boxes.view(B, O, 4), None
+        masks = None
+        if self.mask_net is not None:
+            masks = self.masks_from_vecs(obj_vecs)
+            masks = masks.view(B, O, masks.shape[1], masks.shape[2])
+        return obj_vecs.view(B, O, -1), boxes.view(B, O, 4), masks
 
     def forward_ragged(self, objs, triplets, triplet_type, tri_off, obj_off):
         """Flat interface: objs [NO,A], triplets [NT,3] (graph-local ids), triplet_type [NT], offsets [B+1] i32

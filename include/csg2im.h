@@ -325,6 +325,41 @@ int csg_head_fwd(const void* h, int ldh, const float* w, const float* b, int M, 
 size_t csg_head_bwd_workspace(int M, int K, int nout);
 int csg_head_bwd(const float* dy, const void* h, int ldh, const float* w, int M, int K, int nout, void* dh, int lddh,
                  float* dw, float* db, int h_fp16, void* workspace, size_t workspace_bytes, csg_stream_t stream);
+/* The same head for any element format of h / dh (fmt: 0 fp32, 1 bf16, 2 fp16) and with an optional sigmoid: the 1x1
+ * output convolution of the mask head (model.py:62-75).  sigmoid = 1: y = sigmoid(h w^T + b); the backward then takes
+ * those outputs as y (NULL: no sigmoid) and folds sigmoid' = y (1 - y) into dy.  relu = 1: h is a ReLU output and dh
+ * takes its mask (h > 0); relu = 0: dh = dy w.  Reductions as above, in two ordered levels for many rows. */
+int csg_head_fwd_ex(const void* h, int ldh, int h_fmt, const float* w, const float* b, int M, int K, int nout,
+                    int sigmoid, float* y, csg_stream_t stream);
+size_t csg_head_bwd_ex_workspace(int M, int K, int nout);
+int csg_head_bwd_ex(const float* dy, const float* y, const void* h, int ldh, int h_fmt, const float* w, int M, int K,
+                    int nout, void* dh, int lddh, int dh_fmt, int relu, float* dw, float* db, void* workspace,
+                    size_t workspace_bytes, csg_stream_t stream);
+
+/* ---- mask head of Sg2LayoutModel (sg2im/model.py:62-75, mask_size > 0): per stage Upsample(2) -> BatchNorm2d(C) ->
+ *      Conv2d(C, C, 3, padding=1) -> ReLU, each convolution one GEMM (csg_gemm_bf16 / csg_gemm_f32) over a patch matrix.
+ *      A stage input of side s is x [O*s*s, C] (NHWC rows, row (o*s + y)*s + x); fmt: 0 fp32, 1 bf16, 2 fp16.  BatchNorm
+ *      runs at low resolution (nearest upsampling leaves the batch mean and biased variance unchanged). -------------- */
+/* n = O*s*s rows.  training: batch statistics (deterministic), running_mean / running_var (may be NULL) updated with
+ * `momentum` and the unbiased variance of the 4n upsampled elements, *num_batches_tracked += 1 (also for n = 0, which
+ * leaves the running buffers unchanged).  eval: the running buffers.  Writes mean, invstd and scale = gamma * invstd
+ * [C] (nothing for n = 0). */
+size_t csg_mask_bn_fwd_workspace(int n, int C);
+int csg_mask_bn_fwd(const void* x, int x_fmt, int n, int C, const float* gamma, float* running_mean, float* running_var,
+                    long long* num_batches_tracked, double momentum, double eps, int training, float* scale, float* mean,
+                    float* invstd, void* workspace, size_t workspace_bytes, csg_stream_t stream);
+/* A [O*(2s)^2, 9C] (16-byte aligned) = patches of the upsampled, normalised, zero-padded input:
+ * A[(o*S + Y)*S + X, c*9 + ky*3 + kx] = (x[o, (Y+ky-1)/2, (X+kx-1)/2, c] - mean[c]) * scale[c] + beta[c] inside the
+ * S x S image (S = 2s), 0 outside.  conv.weight.view(C, 9C) is the matching GEMM operand.  C % 8 == 0. */
+int csg_mask_patch(const void* x, int x_fmt, int O, int s, int C, const float* mean, const float* scale,
+                   const float* beta, void* A, int a_fmt, csg_stream_t stream);
+/* Backward of csg_mask_patch and of the BatchNorm in front of it: dA [O*(2s)^2, 9C] -> dx [O*s*s, C] (times (x > 0)
+ * when relu_mask: x is then the previous stage's ReLU output), dgamma, dbeta [C].  mean / invstd from csg_mask_bn_fwd;
+ * training selects the batch-statistics backward.  Deterministic. */
+size_t csg_mask_bn_bwd_workspace(int n, int C);
+int csg_mask_bn_bwd(const void* dA, int da_fmt, const void* x, int x_fmt, int O, int s, int C, const float* gamma,
+                    const float* mean, const float* invstd, int training, int relu_mask, void* dx, int dx_fmt,
+                    float* dgamma, float* dbeta, void* workspace, size_t workspace_bytes, csg_stream_t stream);
 
 /* Multi-tensor Adam (torch.optim.Adam arithmetic, amsgrad off): updates `count` fp32 tensors in place in
  * ceil(count / 48) launches.  params / grads / exp_avg / exp_avg_sq / numel are HOST arrays (device pointers, element
