@@ -20,6 +20,8 @@
 //             factor changes.
 //   generic   the previous tile/butterfly backward is kept for shapes the ring cannot serve (W % 64, H*W % 256,
 //             D % 32 or unaligned gradients).
+//   backward, d masks with fixed boxes (the predicted-mask training step): band-tiled, one more read of the gradient per
+//             chunk of objects (layout_bwd_dmasks_kernel below, csg_layout_bwd_vecs_masks).
 //
 // The pixel weight of object o is separable for boxes_to_layout, S_o(y, x) = ay_o(y) * ax_o(x), and a 4-tap
 // bilinear read of the mask for masks_to_layout.
@@ -1215,6 +1217,266 @@ size_t workspace_bytes(int NO, int D, int H, int W) {
 
 }  // namespace gen
 
+// ========================================================================================
+// backward wrt float masks (masks_to_layout, the training step with predicted masks), band-tiled:
+//   dmasks[o, a, b] = sum_{y, x} G_o(y, x) * wy_o(y, a) * wx_o(x, b),   G_o(y, x) = sum_d dout[n, d, y, x] * vecs[o, d]
+// A CTA owns (image, range of 256-pixel bands) and reads the gradient of its range once per chunk of lcap objects
+// (every channel of a pixel by the same thread), whatever the number of objects covering a pixel: thread = pixel,
+// G of up to LC objects in registers, then per-row tap-column sums T[r][b] = sum_x G(y_r, x) wx(x, b) and their fold
+// along y into per-(range, object) partials in shared memory, in a fixed order.  A second pass sums each object's
+// partials over the ranges its rows meet, in ascending order.  No atomics on floats: runs are bitwise reproducible,
+// and a 16-bit gradient gives exactly the result of its fp32 widening.  The weights of an object's taps come from
+// the sample coordinates of bw::layout_tables_kernel (the ring kernel's tables).
+// ========================================================================================
+namespace dm {
+
+constexpr int NTHREADS = bw::BAND;     // thread = pixel of the current band
+constexpr int LC = 16;                 // objects whose G a thread holds in registers at a time
+constexpr int M_MAX = 32;              // mask sizes served (the tables below grow as M^2)
+
+struct Smem {
+  float* vS;     // [lcap][D]      vecs of the chunk's objects
+  float* G;      // [lcap][BAND]   G of the current band
+  float* T;      // [lcap][RPB][M] per-row tap-column sums of the current band
+  float* acc;    // [lcap][M * M]  partial of the CTA's range
+  int* bx;       // [lcap][M][2]   canvas-column range feeding mask column b
+  int* list;     // [lcap]         chunk-local -> global object id
+  int* act;      // [lcap]         chunk-local ids of the objects that touch the current band
+};
+
+__host__ __device__ inline int rows_per_band(int W) { return W >= bw::BAND ? 1 : bw::BAND / W; }
+
+__host__ __device__ inline size_t smem_bytes(int lcap, int D, int W, int M) {
+  return 4 * ((size_t)lcap * (D + bw::BAND + rows_per_band(W) * M + M * M + 2 * M + 2)) + 16;
+}
+
+__device__ __forceinline__ Smem carve(float* base, int lcap, int D, int W, int M) {
+  Smem s;
+  s.vS = base;
+  s.G = s.vS + (size_t)lcap * D;
+  s.T = s.G + (size_t)lcap * bw::BAND;
+  s.acc = s.T + (size_t)lcap * rows_per_band(W) * M;
+  s.bx = reinterpret_cast<int*>(s.acc + (size_t)lcap * M * M);
+  s.list = s.bx + (size_t)lcap * M * 2;
+  s.act = s.list + lcap;
+  return s;
+}
+
+struct Params {
+  LayoutParams p;
+  const void* dout;      // float, __nv_bfloat16 or __half (the kernel's T)
+  float* partial;        // [splits][NO][M * M]
+  const float* axg;      // [NO][W] column sample coordinates   (bw::layout_tables_kernel<true>)
+  const float* ayg;      // [NO][H] row sample coordinates
+  const int* rng;        // [NO][4] xmin, xmax, ymin, ymax of the non-zero weights
+  int NO, splits, bands_per_item;
+};
+
+// Does object o (table row r4, not poisoned) take part in the rows [ylo, yhi]?  The same test picks the objects of a
+// CTA and the ranges the sum pass reads, so every partial that is read was written.
+__device__ __forceinline__ bool takes_part(int4 r4, int ylo, int yhi) {
+  return r4.x <= r4.y && r4.z <= yhi && r4.w >= ylo;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(NTHREADS, 4) layout_bwd_dmasks_kernel(Params q) {
+  CSG_PDL_WAIT();
+  extern __shared__ __align__(16) float smem_raw[];
+  __shared__ int s_cursor, s_count, s_na;
+  const LayoutParams& p = q.p;
+  const int S = p.M, MM = S * S;
+  const Smem s = carve(smem_raw, p.lcap, p.D, p.W, S);
+  const int tid = threadIdx.x, lane = tid & 31;
+  const int split = blockIdx.x % q.splits, n = blockIdx.x / q.splits;
+  const int obeg = p.obj_off[n], oend = p.obj_off[n + 1];
+  const int ncols = min(p.W, bw::BAND), RPB = rows_per_band(p.W);
+  const int b0 = split * q.bands_per_item;
+  const int row0 = b0 * bw::BAND / p.W;
+  const int row1 = ((b0 + q.bands_per_item) * bw::BAND - 1) / p.W;
+  const size_t plane = (size_t)p.H * p.W;
+  const T* dimg = static_cast<const T*>(q.dout) + (size_t)n * p.D * plane;
+  if (tid == 0) s_cursor = obeg;
+  __syncthreads();
+  while (true) {
+    // the next chunk of objects of image n that take part in the CTA's rows, in ascending order
+    if (tid < 32) {
+      int cursor = s_cursor, count = 0;
+      while (cursor < oend && count < p.lcap) {
+        const int o = cursor + lane;
+        bool keep = false;
+        if (o < oend)
+          keep = !box_poison(ld_f4(p.boxes + 4 * (size_t)o)) &&
+                 takes_part(*reinterpret_cast<const int4*>(q.rng + 4 * (size_t)o), row0, row1);
+        const unsigned bal = __ballot_sync(0xffffffffu, keep);
+        const int pos = count + __popc(bal & ((1u << lane) - 1u));
+        if (__popc(bal) <= p.lcap - count) {
+          if (keep) s.list[pos] = o;
+          count += __popc(bal);
+          cursor += 32;
+        } else {
+          if (keep && pos < p.lcap) s.list[pos] = o;
+          const unsigned last = __ballot_sync(0xffffffffu, keep && pos == p.lcap - 1);
+          cursor += __ffs(last);
+          count = p.lcap;
+        }
+      }
+      if (lane == 0) { s_cursor = min(cursor, oend); s_count = count; }
+    }
+    __syncthreads();
+    const int L = s_count;
+    const bool more = s_cursor < oend;
+    if (L == 0) break;
+    for (int i = tid; i < L * (p.D >> 2); i += NTHREADS) {
+      const int c = i / (p.D >> 2), d4 = i % (p.D >> 2);
+      st_f4(s.vS + c * p.D + d4 * 4, ld_f4(p.vecs + (size_t)s.list[c] * p.D + d4 * 4));
+    }
+    for (int i = tid; i < L * MM; i += NTHREADS) s.acc[i] = 0.f;
+    for (int i = tid; i < L * S; i += NTHREADS) { s.bx[2 * i] = p.W; s.bx[2 * i + 1] = -1; }
+    __syncthreads();
+    for (int i = tid; i < L * p.W; i += NTHREADS) {
+      const int c = i / p.W, x = i % p.W;
+      const Tap t = coord_tap(__ldg(q.axg + (size_t)s.list[c] * p.W + x), S);
+      if (t.i0 >= 0 && t.i0 < S) { atomicMin(&s.bx[(c * S + t.i0) * 2], x); atomicMax(&s.bx[(c * S + t.i0) * 2 + 1], x); }
+      if (t.i0 + 1 >= 0 && t.i0 + 1 < S) {
+        atomicMin(&s.bx[(c * S + t.i0 + 1) * 2], x); atomicMax(&s.bx[(c * S + t.i0 + 1) * 2 + 1], x);
+      }
+    }
+    __syncthreads();
+
+    for (int bb = b0; bb < b0 + q.bands_per_item; ++bb) {
+      const int bpix = bb * bw::BAND;
+      const int y0 = bpix / p.W, x0 = bpix % p.W;
+      // objects of the chunk that touch this band
+      if (tid < 32) {
+        int na = 0;
+        for (int c0 = 0; c0 < L; c0 += 32) {
+          const int c = c0 + lane;
+          bool keep = false;
+          if (c < L) {
+            const int4 r4 = *reinterpret_cast<const int4*>(q.rng + 4 * (size_t)s.list[c]);
+            keep = r4.z <= y0 + RPB - 1 && r4.w >= y0 && r4.x <= x0 + ncols - 1 && r4.y >= x0;
+          }
+          const unsigned bal = __ballot_sync(0xffffffffu, keep);
+          if (keep) s.act[na + __popc(bal & ((1u << lane) - 1u))] = c;
+          na += __popc(bal);
+        }
+        if (lane == 0) s_na = na;
+      }
+      __syncthreads();
+      const int na = s_na;
+      // G of this thread's pixel for LC objects at a time: every channel of the pixel, read in ascending order
+      const T* src = dimg + (size_t)bpix + tid;
+      for (int k0 = 0; k0 < na; k0 += LC) {
+        float g_acc[LC];
+#pragma unroll
+        for (int k = 0; k < LC; ++k) g_acc[k] = 0.f;
+        // (unrolled: 16 gradient loads of the thread in flight, not 4)
+#pragma unroll 4
+        for (int d = 0; d < p.D; d += 4) {
+          const float g0 = to_f32(src[(size_t)d * plane]), g1 = to_f32(src[(size_t)(d + 1) * plane]);
+          const float g2 = to_f32(src[(size_t)(d + 2) * plane]), g3 = to_f32(src[(size_t)(d + 3) * plane]);
+#pragma unroll
+          for (int k = 0; k < LC; ++k) {
+            if (k0 + k < na) {
+              const float4 v = ld_f4(s.vS + s.act[k0 + k] * p.D + d);
+              float a = g_acc[k];
+              a = fmaf(g0, v.x, a); a = fmaf(g1, v.y, a); a = fmaf(g2, v.z, a); a = fmaf(g3, v.w, a);
+              g_acc[k] = a;
+            }
+          }
+        }
+#pragma unroll
+        for (int k = 0; k < LC; ++k)
+          if (k0 + k < na) s.G[(k0 + k) * bw::BAND + tid] = g_acc[k];
+      }
+      __syncthreads();
+      // per-row tap-column sums, (k, r, b) per thread item
+      for (int i = tid; i < na * RPB * S; i += NTHREADS) {
+        const int k = i / (RPB * S), r = (i / S) % RPB, b = i % S;
+        const int c = s.act[k];
+        const float* ax = q.axg + (size_t)s.list[c] * p.W;
+        const float* gr = s.G + k * bw::BAND + r * ncols - x0;
+        const int xlo = max(s.bx[(c * S + b) * 2], x0), xhi = min(s.bx[(c * S + b) * 2 + 1], x0 + ncols - 1);
+        float sum = 0.f;
+        for (int x = xlo; x <= xhi; ++x) {
+          const Tap t = coord_tap(__ldg(ax + x), S);
+          const float w = t.i0 == b ? t.w0 : (t.i0 + 1 == b ? t.w1 : 0.f);
+          sum = fmaf(gr[x], w, sum);
+        }
+        s.T[(k * RPB + r) * S + b] = sum;
+      }
+      __syncthreads();
+      // fold along y into the range's partial (rows in ascending order, bands in ascending order)
+      for (int i = tid; i < na * MM; i += NTHREADS) {
+        const int k = i / MM, a = (i / S) % S, b = i % S;
+        const int c = s.act[k];
+        const float* ay = q.ayg + (size_t)s.list[c] * p.H + y0;
+        float sum = 0.f;
+        for (int r = 0; r < RPB; ++r) {
+          const Tap t = coord_tap(__ldg(ay + r), S);
+          const float w = t.i0 == a ? t.w0 : (t.i0 + 1 == a ? t.w1 : 0.f);
+          sum = fmaf(w, s.T[(k * RPB + r) * S + b], sum);
+        }
+        s.acc[c * MM + a * S + b] += sum;
+      }
+      __syncthreads();
+    }
+    for (int i = tid; i < L * MM; i += NTHREADS) {
+      const int c = i / MM;
+      q.partial[((size_t)split * q.NO + s.list[c]) * MM + i % MM] = s.acc[i];
+    }
+    __syncthreads();
+    if (!more) break;
+  }
+}
+
+// dmasks[o] = sum of o's partials over the ranges its rows meet, ascending; NaN for a poisoned box, exact zeros for an
+// object that touches nothing (the __image__ dummy, box -1)
+__global__ void layout_bwd_dmasks_sum_kernel(const float* __restrict__ partial, const int* __restrict__ rng,
+                                             const float* __restrict__ boxes, float* __restrict__ dmasks, int NO, int MM,
+                                             int splits, int rows_per_split) {
+  CSG_PDL_WAIT();
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (long long)NO * MM) return;
+  const int o = (int)(i / MM), j = (int)(i % MM);
+  if (box_poison(ld_f4(boxes + 4 * (size_t)o))) { dmasks[i] = __int_as_float(0x7fc00000); return; }
+  const int4 r4 = *reinterpret_cast<const int4*>(rng + 4 * (size_t)o);
+  float acc = 0.f;
+  if (r4.x <= r4.y && r4.z <= r4.w)
+    for (int sp = r4.z / rows_per_split; sp <= min(r4.w / rows_per_split, splits - 1); ++sp)
+      acc += partial[((size_t)sp * NO + o) * MM + j];
+  dmasks[i] = acc;
+}
+
+int pick_lcap(int D, int W, int M) {
+  int lcap = 16;
+  while (lcap > 4 && smem_bytes(lcap, D, W, M) > 64 * 1024) lcap -= 4;
+  return lcap;
+}
+
+// ranges per image: ~4 CTAs per SM in all, fewer when the partials would pass 64 MB
+int pick_splits(int N, int NO, int H, int W, int M) {
+  const int nbands = H * W / bw::BAND;
+  int s = 1;
+  // (a range is whole rows: W > 256 takes several bands per row)
+  while (s * 2 <= nbands && nbands % (s * 2) == 0 && ((nbands / (s * 2)) * bw::BAND) % W == 0 &&
+         (long long)N * s < 4LL * csg_num_sms())
+    s *= 2;
+  while (s > 1 && (size_t)s * NO * M * M * 4 > ((size_t)64 << 20)) s /= 2;
+  return s;
+}
+
+bool shape_ok(int D, int H, int W, int M) {
+  return bw::shape_ok(D, H, W) && (W == 64 || W == 128 || W % bw::BAND == 0) && M >= 1 && M <= M_MAX &&
+         smem_bytes(4, D, W, M) <= 200 * 1024;
+}
+
+size_t partial_bytes(int N, int NO, int H, int W, int M) {
+  return (size_t)pick_splits(N, NO, H, W, M) * NO * M * M * 4;
+}
+
+}  // namespace dm
+
 int fill_params(LayoutParams& p, const float* vecs, const float* boxes, const float* masks, const int* obj_off,
                 const float* lin_x, const float* lin_y, int N, int D, int H, int W, int M, int align) {
   CSG_REQUIRE(N >= 0 && D > 0 && H > 0 && W > 0, "layout: bad sizes N=%d D=%d H=%d W=%d", N, D, H, W);
@@ -1274,7 +1536,10 @@ int layout_fwd(const float* vecs, const float* boxes, const float* masks, const 
 template <typename T>
 int layout_bwd_vecs(const T* dout, const float* boxes, const float* masks, const int* obj_off, const float* lin_x,
                     const float* lin_y, float* dvecs, int N, int NO, int D, int H, int W, int M, int align_corners,
-                    int max_objs_per_image, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+                    int max_objs_per_image, void* workspace, size_t workspace_bytes, cudaStream_t stream,
+                    const float** ring_tables = nullptr) {
+  // ring_tables: set to the per-object tables (axg [NO][W], ayg [NO][H], rng [NO][4], contiguous) when the ring or
+  // column-sum kernel ran, left alone otherwise
   LayoutParams p;
   if (int rc = fill_params(p, nullptr, boxes, masks, obj_off, lin_x, lin_y, N, D, H, W, M, align_corners)) return rc;
   if (N == 0 || NO == 0) return 0;
@@ -1319,6 +1584,7 @@ int layout_bwd_vecs(const T* dout, const float* boxes, const float* masks, const
     if (masks) { CSG_CUDA(csg_launch_pdl(bw::layout_tables_kernel<true>, dim3(NO), dim3(128), 0, stream, q.p, NO, axg, ayg, rng)); }
     else       { CSG_CUDA(csg_launch_pdl(bw::layout_tables_kernel<false>, dim3(NO), dim3(128), 0, stream, q.p, NO, axg, ayg, rng)); }
     CSG_CHECK_LAUNCH("csg_layout_bwd_vecs tables");
+    if (ring_tables) *ring_tables = axg;
     const int grid = N * q.cblocks * q.splits;
     const int RR = q.bands_per_item * bw::BAND / W;       // rows per CTA
     if (want_cs && RR <= bw::cs::RR_MAX) {
@@ -1374,6 +1640,91 @@ int layout_bwd_vecs(const T* dout, const float* boxes, const float* masks, const
   return 0;
 }
 
+size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
+
+}  // namespace
+
+CSG_API size_t csg_layout_bwd_geom_workspace(int NO);
+CSG_API int csg_layout_bwd_geom(const float* dout, const float* vecs, const float* boxes, const float* masks,
+                                const int* obj_off, const float* lin_x, const float* lin_y, float* dboxes,
+                                float* dmasks, int N, int NO, int D, int H, int W, int M, int align_corners,
+                                void* workspace, size_t workspace_bytes, cudaStream_t stream);
+CSG_API int csg_layout_bwd_geom_bf16(const void* dout, const float* vecs, const float* boxes, const float* masks,
+                                     const int* obj_off, const float* lin_x, const float* lin_y, float* dboxes,
+                                     float* dmasks, int N, int NO, int D, int H, int W, int M, int align_corners,
+                                     int fp16, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+
+CSG_API size_t csg_layout_bwd_vecs_masks_workspace(int N, int NO, int D, int H, int W, int M) {
+  const size_t vecs = align256(csg_layout_bwd_vecs_workspace(N, NO, D, H, W));
+  size_t rest = align256((size_t)NO * 16) + csg_layout_bwd_geom_workspace(NO);       // shapes served by ring + geom
+  if (dm::shape_ok(D, H, W, M)) {
+    const size_t band = align256((size_t)NO * (W + H + 4) * 4) + dm::partial_bytes(N, NO, H, W, M);
+    if (band > rest) rest = band;
+  }
+  return vecs + rest;
+}
+
+namespace {
+// csg_layout_bwd_vecs_masks with an incoming gradient of element type T
+template <typename T>
+int layout_bwd_vecs_masks(const T* dout, const float* vecs, const float* boxes, const float* masks, const int* obj_off,
+                          const float* lin_x, const float* lin_y, float* dvecs, float* dmasks, int N, int NO, int D,
+                          int H, int W, int M, int align_corners, int max_objs_per_image, void* workspace,
+                          size_t workspace_bytes, cudaStream_t stream) {
+  CSG_REQUIRE(masks != nullptr && M > 0, "layout bwd vecs+masks: float masks are required");
+  CSG_REQUIRE(vecs != nullptr && dvecs != nullptr && dmasks != nullptr, "layout bwd vecs+masks: null vecs / dvecs / dmasks");
+  CSG_REQUIRE(workspace_bytes >= csg_layout_bwd_vecs_masks_workspace(N, NO, D, H, W, M),
+              "layout bwd vecs+masks: workspace too small");
+  if (N == 0 || NO == 0) return 0;
+  char* ws = static_cast<char*>(workspace);
+  const size_t vb = align256(csg_layout_bwd_vecs_workspace(N, NO, D, H, W));
+  const float* tables = nullptr;
+  // d vecs: exactly csg_layout_bwd_vecs
+  if (int rc = layout_bwd_vecs(dout, boxes, masks, obj_off, lin_x, lin_y, dvecs, N, NO, D, H, W, M, align_corners,
+                               max_objs_per_image, ws, vb, stream, &tables))
+    return rc;
+  char* rest = ws + vb;
+  if (!dm::shape_ok(D, H, W, M) || !bw::eligible(dout, D, H, W)) {
+    // shapes the ring kernel does not serve: d masks from the per-object kernel (layout_geom.cu), as before
+    float* dboxes = reinterpret_cast<float*>(rest);
+    void* gws = rest + align256((size_t)NO * 16);
+    const size_t gbytes = csg_layout_bwd_geom_workspace(NO);
+    if constexpr (sizeof(T) == 4)
+      return csg_layout_bwd_geom(dout, vecs, boxes, masks, obj_off, lin_x, lin_y, dboxes, dmasks, N, NO, D, H, W, M,
+                                 align_corners, gws, gbytes, stream);
+    else
+      return csg_layout_bwd_geom_bf16(dout, vecs, boxes, masks, obj_off, lin_x, lin_y, dboxes, dmasks, N, NO, D, H, W,
+                                      M, align_corners, (int)std::is_same<T, __half>::value, gws, gbytes, stream);
+  }
+  dm::Params q;
+  if (int rc = fill_params(q.p, vecs, boxes, masks, obj_off, lin_x, lin_y, N, D, H, W, M, align_corners)) return rc;
+  q.p.TW = W; q.p.TH = H; q.p.tiles_x = q.p.tiles_y = 1;
+  float* own = reinterpret_cast<float*>(rest);
+  if (!tables) {
+    // the ring kernel did not run (CSG_LAYOUT_BWD forced another d vecs path): the same tables, here
+    CSG_CUDA(csg_launch_pdl(bw::layout_tables_kernel<true>, dim3(NO), dim3(128), 0, stream, q.p, NO, own,
+                            own + (size_t)NO * W, reinterpret_cast<int*>(own + (size_t)NO * (W + H))));
+    CSG_CHECK_LAUNCH("csg_layout_bwd_vecs_masks tables");
+    tables = own;
+  }
+  q.dout = dout;
+  q.partial = reinterpret_cast<float*>(rest + align256((size_t)NO * (W + H + 4) * 4));
+  q.axg = tables; q.ayg = tables + (size_t)NO * W; q.rng = reinterpret_cast<const int*>(tables + (size_t)NO * (W + H));
+  q.NO = NO;
+  q.splits = dm::pick_splits(N, NO, H, W, M);
+  q.bands_per_item = H * W / bw::BAND / q.splits;
+  q.p.lcap = dm::pick_lcap(D, W, M);
+  const size_t smem = dm::smem_bytes(q.p.lcap, D, W, M);
+  if (int rc = set_smem(dm::layout_bwd_dmasks_kernel<T>, smem)) return rc;
+  CSG_CUDA(csg_launch_pdl(dm::layout_bwd_dmasks_kernel<T>, dim3(N * q.splits), dim3(dm::NTHREADS), smem, stream, q));
+  CSG_CHECK_LAUNCH("csg_layout_bwd_vecs_masks dmasks");
+  const long long n = (long long)NO * M * M;
+  CSG_CUDA(csg_launch_pdl(dm::layout_bwd_dmasks_sum_kernel, dim3(csg_div_up(n, 256)), dim3(256), 0, stream,
+                          (const float*)q.partial, q.rng, boxes, dmasks, NO, M * M, q.splits,
+                          q.bands_per_item * bw::BAND / W));
+  CSG_CHECK_LAUNCH("csg_layout_bwd_vecs_masks sum");
+  return 0;
+}
 }  // namespace
 
 // ----------------------------------------------------------------------------------------
@@ -1426,4 +1777,27 @@ CSG_API int csg_layout_bwd_vecs_bf16(const void* dout, const float* boxes, const
                            M, align_corners, max_objs_per_image, workspace, workspace_bytes, stream);
   return layout_bwd_vecs(static_cast<const __nv_bfloat16*>(dout), boxes, masks, obj_off, lin_x, lin_y, dvecs, N, NO, D,
                          H, W, M, align_corners, max_objs_per_image, workspace, workspace_bytes, stream);
+}
+
+CSG_API int csg_layout_bwd_vecs_masks(const float* dout, const float* vecs, const float* boxes, const float* masks,
+                                      const int* obj_off, const float* lin_x, const float* lin_y, float* dvecs,
+                                      float* dmasks, int N, int NO, int D, int H, int W, int M, int align_corners,
+                                      int max_objs_per_image, void* workspace, size_t workspace_bytes,
+                                      cudaStream_t stream) {
+  return layout_bwd_vecs_masks(dout, vecs, boxes, masks, obj_off, lin_x, lin_y, dvecs, dmasks, N, NO, D, H, W, M,
+                               align_corners, max_objs_per_image, workspace, workspace_bytes, stream);
+}
+
+CSG_API int csg_layout_bwd_vecs_masks_bf16(const void* dout, const float* vecs, const float* boxes, const float* masks,
+                                           const int* obj_off, const float* lin_x, const float* lin_y, float* dvecs,
+                                           float* dmasks, int N, int NO, int D, int H, int W, int M, int align_corners,
+                                           int max_objs_per_image, int fp16, void* workspace, size_t workspace_bytes,
+                                           cudaStream_t stream) {
+  if (fp16)
+    return layout_bwd_vecs_masks(static_cast<const __half*>(dout), vecs, boxes, masks, obj_off, lin_x, lin_y, dvecs,
+                                 dmasks, N, NO, D, H, W, M, align_corners, max_objs_per_image, workspace,
+                                 workspace_bytes, stream);
+  return layout_bwd_vecs_masks(static_cast<const __nv_bfloat16*>(dout), vecs, boxes, masks, obj_off, lin_x, lin_y,
+                               dvecs, dmasks, N, NO, D, H, W, M, align_corners, max_objs_per_image, workspace,
+                               workspace_bytes, stream);
 }

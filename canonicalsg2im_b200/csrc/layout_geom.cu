@@ -10,7 +10,9 @@
 //     once (g = sum_d dout * vec), and accumulates the box / mask-tap gradients in double in a fixed order.
 //
 // Both are HBM-light compared with the training compositor (layout.cu); they exist for completeness of the
-// drop-in (inference canvases, predicted-mask training), and are deterministic.
+// drop-in (inference canvases, box gradients), and are deterministic.  The predicted-mask training step takes d masks
+// from the band-tiled kernel of layout.cu (csg_layout_bwd_vecs_masks), which falls back to this one on shapes the ring
+// kernel does not serve.
 #include "layout_common.cuh"
 
 namespace {

@@ -42,12 +42,16 @@ def cast_bf16(w, transpose=False):
     return out
 
 
-def cast_bf16_multi(jobs, dtype=BF):
-    """jobs: list of (fp32 matrix, transpose) -> list of bf16 (or fp16) copies, one launch."""
+def cast_bf16_multi(jobs, dtype=BF, outs=None):
+    """jobs: list of (fp32 matrix, transpose) -> list of bf16 (or fp16) copies, one launch.  ``outs``: cast into these
+    tensors (contiguous, of the copies' shapes and ``dtype``) instead of new ones."""
     import ctypes
     srcs = [f32c(w) for w, _ in jobs]
-    outs = [torch.empty((w.shape[1], w.shape[0]) if tr else tuple(w.shape), dtype=dtype, device=w.device)
-            for w, (_, tr) in zip(srcs, jobs)]
+    shapes = [(w.shape[1], w.shape[0]) if tr else tuple(w.shape) for w, (_, tr) in zip(srcs, jobs)]
+    if outs is None:
+        outs = [torch.empty(shp, dtype=dtype, device=w.device) for w, shp in zip(srcs, shapes)]
+    elif any(tuple(o.shape) != tuple(shp) or o.dtype != dtype or not o.is_contiguous() for o, shp in zip(outs, shapes)):
+        raise ValueError("cast_bf16_multi: outs do not match the copies' shapes / dtype")
     n = len(jobs)
     VP, IA = ctypes.c_void_p * n, ctypes.c_int * n
     rc = lib().csg_cast_bf16_multi(n, VP(*[w.data_ptr() for w in srcs]), VP(*[o.data_ptr() for o in outs]),

@@ -93,6 +93,21 @@ class _LayoutFn(torch.autograd.Function):
         dvecs = dboxes = dmasks = None
         L = lib()
         lin_x, lin_y = ctx.lin
+        want_dm = ctx.needs_input_grad[2] and ctx.masks_float
+        if ctx.needs_input_grad[0] and want_dm and not ctx.needs_input_grad[1]:
+            # predicted masks on fixed boxes (the training step with a mask head): d vecs and d masks from one entry
+            # point, d masks band-tiled instead of one pass over the gradient per object
+            dvecs = torch.empty((NO, D), dtype=torch.float32, device=dout.device)
+            dmasks = torch.empty_like(masks)
+            ws = workspace(L.csg_layout_bwd_vecs_masks_workspace(N, NO, D, H, W, M), dout.device)
+            args = (ptr(dout), ptr(vecs), ptr(boxes), ptr(masks), ptr(obj_off), ptr(lin_x), ptr(lin_y), ptr(dvecs),
+                    ptr(dmasks), N, NO, D, H, W, M, align, max_objs)
+            if fp16 is None:
+                rc = L.csg_layout_bwd_vecs_masks(*args, ptr(ws), ws.numel(), _stream())
+            else:
+                rc = L.csg_layout_bwd_vecs_masks_bf16(*args, fp16, ptr(ws), ws.numel(), _stream())
+            _lib.check(rc, "csg_layout_bwd_vecs_masks")
+            return dvecs, None, dmasks, None, None, None, None, None, None, None, None
         if ctx.needs_input_grad[0]:
             dvecs = torch.empty((NO, D), dtype=torch.float32, device=dout.device)
             ws = workspace(L.csg_layout_bwd_vecs_workspace(N, NO, D, H, W), dout.device)

@@ -62,28 +62,37 @@ def _stages(net):
 # invalidate_weight_copies below).  A stale or missing entry makes the call cast its weights itself: forgetting
 # refresh_weight_copies costs time, never correctness.
 # ---------------------------------------------------------------------------------------------------------------
-_WCOPIES = {}      # data_ptr of the first 3x3 conv weight -> dict(act, params, versions, copies)
+_WCOPIES = {}      # data_ptr of the first 3x3 conv weight -> dict(act, params, shapes, versions, copies)
 
 
 def _conv_weights(net):
     return [conv.weight for _, conv in _stages(net)[0]]
 
 
-def _cast(weights, act):
+def _cast(weights, act, outs=None):
     from .graph_tc import cast_bf16_multi
     jobs = []
     for w in weights:
         m = w.detach().reshape(w.shape[0], -1)
         jobs += [(m, False), (m, True)]
-    return cast_bf16_multi(jobs, act)
+    return cast_bf16_multi(jobs, act, outs)
 
 
 def refresh_weight_copies(net, act=BF):
-    """Cast the 3x3 convolution weights of ``net`` into their cached 16-bit copies (one launch)."""
+    """Cast the 3x3 convolution weights of ``net`` into their cached 16-bit copies (one launch).  The copies are
+    allocated on first use (or when the weights, their shapes or ``act`` change) and refilled in place afterwards: a
+    captured CUDA graph holds their addresses, so its replays read the copies of the current weights."""
     weights = _conv_weights(net)
     if not weights or any(not w.is_cuda or w.dtype != torch.float32 for w in weights):
         return
-    _WCOPIES[weights[0].data_ptr()] = {"act": act, "params": tuple(weights),
+    e = _WCOPIES.get(weights[0].data_ptr())
+    if (e is not None and e["act"] == act and len(e["params"]) == len(weights)
+            and all(a is b for a, b in zip(e["params"], weights))
+            and all(tuple(a.shape) == tuple(b) for a, b in zip(weights, e["shapes"]))):
+        _cast(weights, act, e["copies"])
+        e["versions"] = tuple(w._version for w in weights)
+        return
+    _WCOPIES[weights[0].data_ptr()] = {"act": act, "params": tuple(weights), "shapes": [tuple(w.shape) for w in weights],
                                        "versions": tuple(w._version for w in weights), "copies": _cast(weights, act)}
 
 

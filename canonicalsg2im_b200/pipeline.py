@@ -8,7 +8,8 @@
 
 As in the reference's training graph the canvas is composited from the GENERATOR's own ``AttributeEmbeddings``
 table (generator.py:16,80), not from the GCN output, so the canvas gradient reaches that table only; the GCN is
-trained by the box loss.  All stages are csg2im kernels; torch provides memory and autograd bookkeeping.
+trained by the box loss.  With ``mask_size > 0`` the canvas is ``masks_to_layout`` with the mask head's PREDICTED masks
+(meta_models.py:48), and its gradient reaches the head and the GCN as well.  All stages are csg2im kernels; torch provides memory and autograd bookkeeping.
 """
 import numpy as np
 import os
@@ -24,14 +25,14 @@ from .optim import FusedAdam
 from .parallel import BucketedGradAllReduce
 
 
-def build_opt(vocab: synth.Vocab, embedding_dim=128, gconv_dim=128, hidden_dim=512, num_layers=5):
+def build_opt(vocab: synth.Vocab, embedding_dim=128, gconv_dim=128, hidden_dim=512, num_layers=5, mask_size=0):
     import argparse
     attrs = {"a%d" % i: {str(j): j for j in range(vocab.num_obj_classes if vocab.num_attributes == 1 else 8)}
              for i in range(vocab.num_attributes)}
     return argparse.Namespace(
         vocab={"attributes": attrs, "pred_idx_to_name": vocab.pred_names, "pred_name_to_idx": vocab.pred_ids},
         embedding_dim=embedding_dim, gconv_dim=gconv_dim, gconv_hidden_dim=hidden_dim, gconv_pooling="avg",
-        gconv_num_layers=num_layers, mlp_normalization="none", mask_size=0, learned_init="uniform")
+        gconv_num_layers=num_layers, mlp_normalization="none", mask_size=mask_size, learned_init="uniform")
 
 
 class HostBatch:
@@ -94,7 +95,7 @@ class HostBatch:
 class SgToLayoutStep:
     def __init__(self, vocab, device, precision="fp32", H=64, W=64, learned_converse=True,
                  learned_transitivity=True, lr=1e-4, seed=0, distributed=False, bbox_pred_loss_weight=10.0,
-                 global_batch=None, use_graph=False, canvas_dtype=torch.float32):
+                 global_batch=None, use_graph=False, canvas_dtype=torch.float32, mask_size=0):
         """``global_batch``: number of graphs of the GLOBAL batch this rank holds a shard of.  The box loss is a mean
         over images (pix2pix_model.py:85), so with shards of unequal graph counts (cost-balanced sharding) every rank
         scales its loss by B_local / B_global and the gradients are SUMMED over ranks: the result equals the
@@ -102,16 +103,29 @@ class SgToLayoutStep:
         gradients are averaged (the reference's DataParallel behaviour, meta_models.py:17).
 
         ``canvas_dtype``: element type of the canvas and of the ``canvas_grad`` that ``step`` takes (``torch.float32``,
-        ``torch.bfloat16`` or ``torch.float16``), e.g. the dtype a mixed-precision generator consumes it in."""
+        ``torch.bfloat16`` or ``torch.float16``), e.g. the dtype a mixed-precision generator consumes it in.
+
+        ``mask_size``: 0 (default) composites the canvas from the GT boxes alone (boxes_to_layout).  A power of two
+        builds the model with its mask head (model.py:62-75) and composites masks_to_layout on the GT boxes with the
+        PREDICTED masks, as the reference trains on datasets without GT masks (meta_models.py:48, VG): the canvas
+        gradient then reaches the generator's embedding, the mask head and, through it, the GCN.  The head's BatchNorm
+        normalises over the rows of the ragged batch (every object of the batch, ``__image__`` dummies included) and
+        updates its running buffers on the device inside the step, so a CUDA-graph replay updates them as an eager
+        step does.  With ``distributed``, the statistics and running buffers are per rank (DataParallel's per-replica
+        behaviour), so ``global_batch`` sharding no longer reproduces the single-GPU gradient of the whole batch."""
         if canvas_dtype not in (torch.float32, torch.bfloat16, torch.float16):
             raise ValueError("canvas_dtype must be torch.float32, torch.bfloat16 or torch.float16")
         self.canvas_dtype = canvas_dtype
         self.vocab, self.device, self.H, self.W = vocab, device, H, W
         self.flags = (learned_converse, learned_transitivity)
-        self.model = Sg2LayoutModel(build_opt(vocab), precision=precision).to(device)
+        self.mask_size = int(mask_size)
+        self.model = Sg2LayoutModel(build_opt(vocab, mask_size=self.mask_size), precision=precision).to(device)
         st = {k: torch.from_numpy(v) for k, v in synth.make_state(vocab, seed=seed).items()}
         for i in range(len(self.model.gconvs)):
             st["gconvs.%d.predicates_transitive_weights" % i] = st["trans_candidates_weights"]
+        if self.mask_size > 0:
+            st.update({k: torch.from_numpy(np.asarray(v)) for k, v in
+                       synth.make_mask_state(self.model.args["gconv_dim"], self.mask_size, seed=seed).items()})
         self.model.load_state_dict(st, strict=True)
         # the generator's own object embedding (generator.py:16), the source of the canvas vectors (generator.py:80)
         opt = build_opt(vocab)
@@ -120,10 +134,13 @@ class SgToLayoutStep:
             {k: torch.from_numpy(v) for k, v in synth.make_layout_state(vocab, opt.embedding_dim, seed=seed).items()},
             strict=True)
         self.bbox_pred_loss_weight = bbox_pred_loss_weight
+        self.last_masks = None         # masks_pred of the last eager forward (mask_size > 0)
         self.refresh_tables()
         # gradient buckets in the order they complete: box_net, gconvs 4..0, then embeddings + shared weights
         layers = list(self.model.gconvs)
         buckets = [list(self.model.box_net.parameters())]
+        if self.model.mask_net is not None:      # the head's gradients are final together with box_net's
+            buckets[0] += list(self.model.mask_net.parameters())
         for layer in reversed(layers):
             buckets.append([p for n, p in layer.named_parameters() if "predicates_transitive_weights" not in n])
         buckets.append(list(self.model.attribute_embedding.parameters()) + list(self.model.pred_embeddings.parameters())
@@ -209,10 +226,21 @@ class SgToLayoutStep:
             branch.wait_stream(main)
         with torch.cuda.stream(branch):
             layout_vecs = self.layout_embedding(d["objs"])
-            canvas = layout_batched(layout_vecs, d["boxes"], d["obj_off"], self.H, self.W,
-                                    max_objs_per_image=d["max_objs"], out_dtype=self.canvas_dtype)
+            if self.mask_size == 0:
+                canvas = layout_batched(layout_vecs, d["boxes"], d["obj_off"], self.H, self.W,
+                                        max_objs_per_image=d["max_objs"], out_dtype=self.canvas_dtype)
         obj_vecs, boxes_pred = self.model.forward_ragged(d["objs"], res.triplets, res.triplet_type, res.tri_off,
                                                          d["obj_off"])
+        if self.mask_size > 0:
+            # predicted masks (meta_models.py:48): the compositor waits for the head; the embedding lookup above stayed
+            # on the branch stream
+            masks_pred = self.model.masks_from_vecs(obj_vecs)
+            if branch is not main:
+                branch.wait_stream(main)
+            with torch.cuda.stream(branch):
+                canvas = layout_batched(layout_vecs, d["boxes"], d["obj_off"], self.H, self.W, masks=masks_pred,
+                                        max_objs_per_image=d["max_objs"], out_dtype=self.canvas_dtype)
+            self.last_masks = masks_pred.detach()
         if branch is not main:
             main.wait_stream(branch)
         weight = self.bbox_pred_loss_weight
@@ -375,10 +403,14 @@ class SgToLayoutInference:
         (layout.py:48-77,135-147), dummy objects removed (utils.py:56-63)
 
     ``step(d)`` expects the device tensors of :class:`HostBatch` plus ``centers [NO, 2]`` and ``masks [NO, M, M]``;
-    the canvas it returns has dtype ``canvas_dtype`` (fp32, or the fp32 canvas rounded once to bf16 / fp16)."""
+    the canvas it returns has dtype ``canvas_dtype`` (fp32, or the fp32 canvas rounded once to bf16 / fp16).
+
+    ``mask_size > 0`` builds the model with its mask head, in eval mode (BatchNorm on its running buffers): a batch
+    without ``masks`` is then composited from the PREDICTED masks (``model.masks_from_vecs(obj_vecs)``, model.py:121-123),
+    a batch with GT masks as before."""
 
     def __init__(self, vocab, device, precision="fp16", H=256, W=256, embedding_dim=32, attr_sizes=None,
-                 learned_converse=True, learned_transitivity=True, seed=0, canvas_dtype=torch.float32):
+                 learned_converse=True, learned_transitivity=True, seed=0, canvas_dtype=torch.float32, mask_size=0):
         import argparse
         if canvas_dtype not in (torch.float32, torch.bfloat16, torch.float16):
             raise ValueError("canvas_dtype must be torch.float32, torch.bfloat16 or torch.float16")
@@ -391,13 +423,19 @@ class SgToLayoutInference:
         opt = argparse.Namespace(
             vocab={"attributes": attrs, "pred_idx_to_name": vocab.pred_names, "pred_name_to_idx": vocab.pred_ids},
             embedding_dim=embedding_dim, gconv_dim=128, gconv_hidden_dim=512, gconv_pooling="avg", gconv_num_layers=5,
-            mlp_normalization="none", mask_size=0, learned_init="uniform")
+            mlp_normalization="none", mask_size=int(mask_size), learned_init="uniform")
+        self.mask_size = int(mask_size)
         self.model = Sg2LayoutModel(opt, precision=precision).to(device)
         st = {k: torch.from_numpy(v) for k, v in
               synth.make_state(vocab, embedding_dim=embedding_dim, seed=seed, attr_vocab_sizes=sizes).items()}
         for i in range(len(self.model.gconvs)):
             st["gconvs.%d.predicates_transitive_weights" % i] = st["trans_candidates_weights"]
+        if self.mask_size > 0:
+            st.update({k: torch.from_numpy(np.asarray(v)) for k, v in
+                       synth.make_mask_state(opt.gconv_dim, self.mask_size, seed=seed).items()})
         self.model.load_state_dict(st, strict=True)
+        if self.mask_size > 0:
+            self.model.eval()
         self.layout_embedding = AttributeEmbeddings(attrs, embedding_dim).to(device)
         self.layout_embedding.load_state_dict(
             {k: torch.from_numpy(v) for k, v in
@@ -428,6 +466,11 @@ class SgToLayoutInference:
         # the __image__ dummy is removed from the canvas (utils.py:56-63): a box of -1 samples nothing
         dummy = (d["objs"][:, :1] == 0)
         boxes = torch.where(dummy, torch.full_like(boxes_pred, -1.0), boxes_pred.float())
-        canvas = layout_batched(self.layout_embedding(d["objs"]), boxes, d["obj_off"], self.H, self.W, masks=d["masks"],
+        masks = d.get("masks")
+        if masks is None:
+            if self.mask_size == 0:
+                raise ValueError("a batch without masks needs a model with a mask head (mask_size > 0)")
+            masks = self.model.masks_from_vecs(obj_vecs)
+        canvas = layout_batched(self.layout_embedding(d["objs"]), boxes, d["obj_off"], self.H, self.W, masks=masks,
                                 test_mode=True, out_dtype=self.canvas_dtype)
         return canvas, boxes_pred, int(res.triplets.shape[0])

@@ -282,3 +282,26 @@ def make_layout_state(vocab: Vocab, embedding_dim=128, seed=0, attr_vocab_sizes=
         st["attribute_fc_gen.weight"] = det_tensor((n, n), k + 1, float(np.sqrt(6.0 / n)))
         st["attribute_fc_gen.bias"] = det_tensor((n,), k + 2, float(1.0 / np.sqrt(n)))
     return st
+
+
+def make_mask_state(gconv_dim=128, mask_size=16, seed=0):
+    """Random-init weights and running buffers of the mask head (``sg2im/model.py:62-75``, ``mask_size > 0``) keyed like
+    ``Sg2LayoutModel``'s state dict (``mask_net.*``).  BatchNorm weights and running variances are uniform in
+    [0.5, 1.5), running means and all biases in [-0.2, 0.2), convolution weights in +-sqrt(3 / fan_in);
+    ``num_batches_tracked`` starts at 0."""
+    from .mask_head import build_mask_net
+    st = {}
+    k = seed * 3001 + 907
+    for name, v in build_mask_net(gconv_dim, mask_size).state_dict().items():
+        k += 1
+        shape = tuple(v.shape)
+        if name.endswith("num_batches_tracked"):
+            st["mask_net." + name] = np.zeros((), np.int64)
+        elif name.endswith("running_var") or (v.dim() == 1 and name.endswith("weight")):
+            st["mask_net." + name] = det_tensor(shape, k, 0.5) + np.float32(1.0)
+        elif name.endswith("running_mean") or name.endswith("bias"):
+            st["mask_net." + name] = det_tensor(shape, k, 0.2)
+        else:
+            fan_in = int(np.prod(shape[1:]))
+            st["mask_net." + name] = det_tensor(shape, k, float(np.sqrt(3.0 / fan_in)))
+    return st

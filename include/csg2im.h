@@ -99,6 +99,23 @@ int csg_layout_bwd_geom_bf16(const void* dout, const float* vecs, const float* b
                              const int* obj_off, const float* lin_x, const float* lin_y, float* dboxes,
                              float* dmasks, int N, int NO, int D, int H, int W, int M, int align_corners,
                              int fp16, void* workspace, size_t workspace_bytes, csg_stream_t stream);
+/* autograd of csg_layout_fwd wrt vecs and float masks [NO,M,M] together, boxes held fixed (the training step with
+ * predicted masks on GT boxes).  dvecs is bitwise that of csg_layout_bwd_vecs.  On shapes the ring kernel serves
+ * (W % 64 == 0 with W = 64, 128 or a multiple of 256, H*W % 256 == 0, D % 32 == 0, M <= 32, 16-byte aligned dout)
+ * dmasks comes from a band-tiled kernel that reads dout once more per chunk of 16 objects (fp32 sums in a fixed
+ * order, deterministic); on other shapes from csg_layout_bwd_geom.  Either way a poisoned box (zero / NaN extent,
+ * non-finite origin) gives a NaN dmasks row and an object that touches no pixel an exact-zero row.  The _bf16 form
+ * takes a bf16 (fp16 = 0) or fp16 (fp16 = 1) gradient, widened on load: results are bitwise those of its widening. */
+size_t csg_layout_bwd_vecs_masks_workspace(int N, int NO, int D, int H, int W, int M);
+int csg_layout_bwd_vecs_masks(const float* dout, const float* vecs, const float* boxes, const float* masks,
+                              const int* obj_off, const float* lin_x, const float* lin_y, float* dvecs,
+                              float* dmasks, int N, int NO, int D, int H, int W, int M, int align_corners,
+                              int max_objs_per_image, void* workspace, size_t workspace_bytes, csg_stream_t stream);
+int csg_layout_bwd_vecs_masks_bf16(const void* dout, const float* vecs, const float* boxes, const float* masks,
+                                   const int* obj_off, const float* lin_x, const float* lin_y, float* dvecs,
+                                   float* dmasks, int N, int NO, int D, int H, int W, int M, int align_corners,
+                                   int max_objs_per_image, int fp16, void* workspace, size_t workspace_bytes,
+                                   csg_stream_t stream);
 
 /* ---- box crops: sg2im/bilinear.py:65-94 (crop_bbox, backend 'cudnn'), :44-62 (crop_bbox_batch_cudnn).
  *      Crops crop_off[n]..crop_off[n+1] sample image n of feats [N,C,H,W] in place (the reference expands the
