@@ -7,7 +7,8 @@
 //                   contiguous range of rows in order, accumulating into a private [V, E] table in shared memory;
 //                   the per-block tables are then summed in block order (torch's embedding backward sorts the
 //                   indices with a radix sort per call and accumulates with atomics);
-//   csg_box_loss    per-image masked smooth-L1 box loss of the generator (bbox_pred_all / bbox_pred) and its gradient.
+//   csg_box_loss    per-image masked smooth-L1 box loss of the generator (bbox_pred_all / bbox_pred) and its gradient;
+//   csg_mask_loss   binary cross-entropy mask loss of the generator (mean over every mask element) and its gradient.
 #include "common.cuh"
 #include <cuda_bf16.h>
 
@@ -214,6 +215,82 @@ __global__ void __launch_bounds__(1024) box_loss_mean_kernel(const float* __rest
   if (threadIdx.x == 0) loss[0] = total / (float)B;
 }
 
+// Mask term of the generator loss, weight * F.binary_cross_entropy(pred, target) (mean over all n elements), with
+// torch's arithmetic: per element -(t max(log p, -100) + (1 - t) max(log(1 - p), -100)) written as torch's CPU kernel
+// writes it, and d/dp = ((weight (p - t)) / max((1 - p) p, 1e-12)) / n, rounded step by step in the same order (the
+// explicit _rn intrinsics keep nvcc from contracting them into FMAs), so a saturated p gives torch's bits: p == 1
+// yields a finite d/dp that sigmoid' = 0 turns into an exact zero.  Block partials of the element losses in double, a
+// fixed grid for a given n, one ordered final pass: two calls are bitwise equal.
+constexpr int ML_THREADS = 256, ML_PER_THREAD = 8, ML_MAX_BLOCKS = 1024;
+int mask_loss_blocks(long long n) {
+  const long long b = (n + ML_THREADS * ML_PER_THREAD - 1) / (ML_THREADS * ML_PER_THREAD);
+  return (int)(b < ML_MAX_BLOCKS ? b : ML_MAX_BLOCKS);
+}
+
+// std::max(a, b) = a < b ? b : a: a NaN first argument is returned (fmaxf would drop it)
+__device__ __forceinline__ float std_max(float a, float b) { return a < b ? b : a; }
+
+__device__ __forceinline__ double block_sum_double(double v, double* red) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  double t = 0.0;
+  if (threadIdx.x < 32) {
+    t = threadIdx.x < (blockDim.x >> 5) ? red[threadIdx.x] : 0.0;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+  }
+  return t;                                            // valid in thread 0
+}
+
+template <bool TARGET_I64>
+__global__ void __launch_bounds__(ML_THREADS) mask_loss_partial_kernel(const float* __restrict__ pred,
+                                                                      const void* __restrict__ target, long long n,
+                                                                      float weight, float* __restrict__ dpred,
+                                                                      double* __restrict__ partial) {
+  CSG_PDL_WAIT();
+  __shared__ double red[ML_THREADS / 32];
+  const long long stride = (long long)gridDim.x * ML_THREADS;
+  const float fn = (float)n;
+  double s = 0.0;
+  for (long long i0 = (long long)blockIdx.x * ML_THREADS + threadIdx.x; i0 < n; i0 += stride * ML_PER_THREAD) {
+    float p[ML_PER_THREAD], t[ML_PER_THREAD];
+#pragma unroll
+    for (int k = 0; k < ML_PER_THREAD; ++k) {        // all loads in flight before the arithmetic
+      const long long i = i0 + k * stride;
+      p[k] = t[k] = 0.f;
+      if (i < n) {
+        p[k] = __ldcs(pred + i);
+        t[k] = TARGET_I64 ? (float)__ldcs(static_cast<const long long*>(target) + i)
+                          : __ldcs(static_cast<const float*>(target) + i);
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < ML_PER_THREAD; ++k) {
+      const long long i = i0 + k * stride;
+      if (i < n) {
+        const float l1 = std_max(log1pf(-p[k]), -100.f), l0 = std_max(logf(p[k]), -100.f);
+        s += (double)__fsub_rn(__fmul_rn(__fsub_rn(t[k], 1.f), l1), __fmul_rn(t[k], l0));
+        const float den = std_max(__fmul_rn(__fsub_rn(1.f, p[k]), p[k]), 1e-12f);
+        __stcs(dpred + i, __fdiv_rn(__fdiv_rn(__fmul_rn(weight, __fsub_rn(p[k], t[k])), den), fn));
+      }
+    }
+  }
+  const double b = block_sum_double(s, red);
+  if (threadIdx.x == 0) partial[blockIdx.x] = b;
+}
+
+// loss[0] = weight * (sum of the block partials in block order / n); blocks == 0 (n == 0) reads nothing and gives 0 / 0
+__global__ void __launch_bounds__(ML_MAX_BLOCKS) mask_loss_final_kernel(const double* __restrict__ partial, int blocks,
+                                                                        long long n, float weight, float* __restrict__ loss) {
+  CSG_PDL_WAIT();
+  __shared__ double red[ML_MAX_BLOCKS / 32];
+  const double v = (int)threadIdx.x < blocks ? partial[threadIdx.x] : 0.0;
+  const double total = block_sum_double(v, red);
+  if (threadIdx.x == 0) loss[0] = __fmul_rn((float)(total / (double)n), weight);
+}
+
 }  // namespace
 
 CSG_API int csg_embed_fwd(const float* table, const long long* idx, long long idx_stride, int n, int V, int E,
@@ -279,5 +356,33 @@ CSG_API int csg_box_loss(const float* pred, const float* gt, const long long* ob
   CSG_CHECK_LAUNCH("csg_box_loss image");
   CSG_CUDA(csg_launch_pdl(box_loss_mean_kernel, dim3(1), dim3(1024), 0, stream, (const float*)loss_all, B, loss));
   CSG_CHECK_LAUNCH("csg_box_loss mean");
+  return 0;
+}
+
+CSG_API size_t csg_mask_loss_workspace(long long n) {
+  return (size_t)(n > 0 ? mask_loss_blocks(n) : 0) * sizeof(double) + 256;
+}
+
+// Mask term of the generator loss (sg2im's compute_generator_loss): loss[0] = weight * F.binary_cross_entropy(pred,
+// target), the mean over n elements, and dpred [n] = d loss[0] / d pred.  target_fmt 0: fp32 targets (soft targets in
+// [0, 1] allowed), 1: int64.  n == 0: loss[0] = NaN (the mean of nothing) and nothing is read.
+CSG_API int csg_mask_loss(const float* pred, const void* target, int target_fmt, long long n, double weight,
+                          float* loss, float* dpred, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  CSG_REQUIRE(n >= 0 && (target_fmt == 0 || target_fmt == 1), "mask_loss: n=%lld target_fmt=%d", n, target_fmt);
+  CSG_REQUIRE(workspace_bytes >= csg_mask_loss_workspace(n), "mask_loss: workspace too small");
+  double* partial = reinterpret_cast<double*>(workspace);
+  const int blocks = n > 0 ? mask_loss_blocks(n) : 0;
+  if (blocks > 0) {
+    if (target_fmt == 1)
+      CSG_CUDA(csg_launch_pdl(mask_loss_partial_kernel<true>, dim3(blocks), dim3(ML_THREADS), 0, stream, pred, target, n,
+                              (float)weight, dpred, partial));
+    else
+      CSG_CUDA(csg_launch_pdl(mask_loss_partial_kernel<false>, dim3(blocks), dim3(ML_THREADS), 0, stream, pred, target,
+                              n, (float)weight, dpred, partial));
+    CSG_CHECK_LAUNCH("csg_mask_loss partial");
+  }
+  CSG_CUDA(csg_launch_pdl(mask_loss_final_kernel, dim3(1), dim3(ML_MAX_BLOCKS), 0, stream, (const double*)partial, blocks,
+                          n, (float)weight, loss));
+  CSG_CHECK_LAUNCH("csg_mask_loss final");
   return 0;
 }

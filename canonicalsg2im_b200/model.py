@@ -99,6 +99,46 @@ def bbox_pred_loss(boxes_pred, boxes, objs, weight=10.0):
     return bbox_pred_loss_ragged(boxes_pred, boxes, objs.reshape(B * O, -1), off, weight)
 
 
+class _MaskLossFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, pred, target, weight):
+        p, n = pred.detach().contiguous(), pred.numel()
+        target = target.contiguous()
+        loss = torch.empty(1, dtype=torch.float32, device=p.device)
+        dpred = torch.empty_like(p)
+        L = lib()
+        ws = workspace(L.csg_mask_loss_workspace(n), p.device)
+        _lib.check(L.csg_mask_loss(ptr(p), ptr(target), int(target.dtype == torch.int64), n, float(weight), ptr(loss),
+                                   ptr(dpred), ptr(ws), ws.numel(), _stream()), "csg_mask_loss")
+        ctx.save_for_backward(dpred)
+        return loss[0]
+
+    @staticmethod
+    def backward(ctx, dloss):
+        (dpred,) = ctx.saved_tensors
+        return dpred * dloss, None, None
+
+
+def mask_pred_loss(masks_pred, masks_gt, weight=1.0):
+    """Mask term of the generator loss on GT masks (sg2im's ``compute_generator_loss``):
+    ``weight * F.binary_cross_entropy(masks_pred, masks_gt.float())``, the mean over every element, with torch's clamps
+    (``log`` at -100, ``(1 - p) p`` at 1e-12 in the gradient).  ``masks_pred`` / ``masks_gt``: any matching shape, e.g.
+    ragged ``[NO, M, M]`` or padded ``[B, O, M, M]``; ``masks_gt`` fp32 (soft targets in [0, 1] allowed) or int64 as the
+    datasets carry them, read without a cast pass; bool, other integer and float dtypes are cast to one of the two.
+    Returns a differentiable scalar; the target gets no gradient.  One pass, no host synchronisation; an empty input
+    gives NaN, as torch's mean of an empty tensor.  Predictions outside [0, 1] are not checked (torch raises)."""
+    need_cuda(masks_pred, masks_gt)
+    if tuple(masks_pred.shape) != tuple(masks_gt.shape):
+        raise ValueError("mask_pred_loss: masks_pred %s and masks_gt %s differ in shape"
+                         % (tuple(masks_pred.shape), tuple(masks_gt.shape)))
+    tgt = masks_gt.detach()
+    if tgt.dtype == torch.bool or tgt.is_floating_point():
+        tgt = tgt.float()
+    else:
+        tgt = tgt.to(torch.int64)
+    return _MaskLossFn.apply(masks_pred.float().reshape(-1), tgt.reshape(-1), weight)
+
+
 def get_conv_converse(model):
     """sg2im/model.py:8-15 — symmetrised converse weights (triu + triu^T)."""
     if isinstance(model, dict):

@@ -9,7 +9,9 @@
 As in the reference's training graph the canvas is composited from the GENERATOR's own ``AttributeEmbeddings``
 table (generator.py:16,80), not from the GCN output, so the canvas gradient reaches that table only; the GCN is
 trained by the box loss.  With ``mask_size > 0`` the canvas is ``masks_to_layout`` with the mask head's PREDICTED masks
-(meta_models.py:48), and its gradient reaches the head and the GCN as well.  All stages are csg2im kernels; torch provides memory and autograd bookkeeping.
+(meta_models.py:48), and its gradient reaches the head and the GCN as well; with ``gt_masks=True`` it is composited from
+the batch's GT masks and the head is trained by the BCE mask term of the generator loss instead.  All stages are
+csg2im kernels; torch provides memory and autograd bookkeeping.
 """
 import numpy as np
 import os
@@ -20,7 +22,7 @@ import torch.nn.functional as F
 from . import synth
 from .canonicalize import canon_count_async, canon_emit, canon_total, converse_tables
 from .layout import layout_batched
-from .model import AttributeEmbeddings, Sg2LayoutModel, bbox_pred_loss_ragged, get_conv_converse
+from .model import AttributeEmbeddings, Sg2LayoutModel, bbox_pred_loss_ragged, get_conv_converse, mask_pred_loss
 from .optim import FusedAdam
 from .parallel import BucketedGradAllReduce
 
@@ -38,7 +40,10 @@ def build_opt(vocab: synth.Vocab, embedding_dim=128, gconv_dim=128, hidden_dim=5
 class HostBatch:
     """Flat host-side batch (pinned when CUDA is available): what a collate function would emit."""
 
-    def __init__(self, graphs, seed=0, pin=True, with_geometry=False, num_uniforms=None):
+    def __init__(self, graphs, seed=0, pin=True, with_geometry=False, num_uniforms=None, with_masks=None):
+        """``with_geometry``: also upload ``centers`` and, when the graphs carry them, ``masks [NO, M, M]`` fp32.
+        ``with_masks``: upload ``masks`` regardless of ``with_geometry`` (True) or never (False); ``None`` = as
+        ``with_geometry`` says (e.g. ``with_masks=True`` alone: the GT-mask training step, which needs no centers)."""
         self.B = len(graphs)
         self.tri_off = np.concatenate([[0], np.cumsum([len(g.triplets) for g in graphs])]).astype(np.int32)
         self.obj_off = np.concatenate([[0], np.cumsum([len(g.objs) for g in graphs])]).astype(np.int32)
@@ -53,8 +58,8 @@ class HostBatch:
         if with_geometry:      # inputs of the on-device graph construction / mask compositor (cfg4)
             arrs["centers"] = np.concatenate([np.concatenate([g.centers, np.zeros((len(g.boxes) - len(g.centers), 2),
                                                                                   np.float32)]) for g in graphs])
-            if graphs[0].masks is not None:
-                arrs["masks"] = np.concatenate([g.masks for g in graphs]).astype(np.float32)
+        if (with_geometry if with_masks is None else with_masks) and graphs[0].masks is not None:
+            arrs["masks"] = np.concatenate([g.masks for g in graphs]).astype(np.float32)
         self.t = {}
         for k, v in arrs.items():
             x = torch.from_numpy(np.ascontiguousarray(v))
@@ -95,7 +100,8 @@ class HostBatch:
 class SgToLayoutStep:
     def __init__(self, vocab, device, precision="fp32", H=64, W=64, learned_converse=True,
                  learned_transitivity=True, lr=1e-4, seed=0, distributed=False, bbox_pred_loss_weight=10.0,
-                 global_batch=None, use_graph=False, canvas_dtype=torch.float32, mask_size=0):
+                 global_batch=None, use_graph=False, canvas_dtype=torch.float32, mask_size=0, gt_masks=False,
+                 mask_loss_weight=1.0):
         """``global_batch``: number of graphs of the GLOBAL batch this rank holds a shard of.  The box loss is a mean
         over images (pix2pix_model.py:85), so with shards of unequal graph counts (cost-balanced sharding) every rank
         scales its loss by B_local / B_global and the gradients are SUMMED over ranks: the result equals the
@@ -112,13 +118,24 @@ class SgToLayoutStep:
         normalises over the rows of the ragged batch (every object of the batch, ``__image__`` dummies included) and
         updates its running buffers on the device inside the step, so a CUDA-graph replay updates them as an eager
         step does.  With ``distributed``, the statistics and running buffers are per rank (DataParallel's per-replica
-        behaviour), so ``global_batch`` sharding no longer reproduces the single-GPU gradient of the whole batch."""
+        behaviour), so ``global_batch`` sharding no longer reproduces the single-GPU gradient of the whole batch.
+
+        ``gt_masks=True`` (needs ``mask_size > 0``): the reference's path for datasets WITH GT masks (COCO).  Every batch
+        carries ``masks [NO, M, M]`` (``HostBatch(..., with_masks=True)``; fp32 or int64); the canvas is masks_to_layout
+        on the GT boxes with those masks (its gradient reaches the generator's embedding only), and the step's loss is
+        the box term plus ``mask_loss_weight * BCE(masks_pred, masks)`` (``model.mask_pred_loss``), which trains the head
+        and, through it, the GCN.  ``mask_loss_weight = 0`` still runs the head's forward (BatchNorm buffers update as in
+        the reference's forward) but adds no term: the head's parameters get no gradient.  With ``global_batch`` the mask
+        term is scaled by B_local / B_global as the box term (not exact: the element count differs per rank)."""
+        if gt_masks and int(mask_size) <= 0:
+            raise ValueError("gt_masks=True needs a mask head (mask_size > 0)")
         if canvas_dtype not in (torch.float32, torch.bfloat16, torch.float16):
             raise ValueError("canvas_dtype must be torch.float32, torch.bfloat16 or torch.float16")
         self.canvas_dtype = canvas_dtype
         self.vocab, self.device, self.H, self.W = vocab, device, H, W
         self.flags = (learned_converse, learned_transitivity)
         self.mask_size = int(mask_size)
+        self.gt_masks, self.mask_loss_weight = bool(gt_masks), float(mask_loss_weight)
         self.model = Sg2LayoutModel(build_opt(vocab, mask_size=self.mask_size), precision=precision).to(device)
         st = {k: torch.from_numpy(v) for k, v in synth.make_state(vocab, seed=seed).items()}
         for i in range(len(self.model.gconvs)):
@@ -135,6 +152,7 @@ class SgToLayoutStep:
             strict=True)
         self.bbox_pred_loss_weight = bbox_pred_loss_weight
         self.last_masks = None         # masks_pred of the last eager forward (mask_size > 0)
+        self.last_mask_loss = None     # mask term of the last eager forward (gt_masks, mask_loss_weight != 0)
         self.refresh_tables()
         # gradient buckets in the order they complete: box_net, gconvs 4..0, then embeddings + shared weights
         layers = list(self.model.gconvs)
@@ -212,6 +230,15 @@ class SgToLayoutStep:
             self.prefetch(d)
         return canon_emit(d.pop("_canon_plan"))
 
+    def _gt_masks(self, d):
+        masks = d.get("masks")
+        if masks is None:
+            raise ValueError("gt_masks=True needs the batch's GT masks d['masks'] [NO, M, M] (HostBatch(with_masks=True))")
+        want = (int(d["objs"].shape[0]), self.mask_size, self.mask_size)
+        if tuple(masks.shape) != want:
+            raise ValueError("d['masks'] is %s, expected %s" % (tuple(masks.shape), want))
+        return masks
+
     def forward(self, d, res):
         # canvas: the generator's own embedding of the objects on the GT boxes (train.py:358, generator.py:80-96).
         # remove_dummy_objects (utils.py:56-63) needs no filtering pass: the __image__ dummy has box -1 and
@@ -220,18 +247,33 @@ class SgToLayoutStep:
         # a node's backward on the stream of its forward, so both the compositor (bandwidth-bound, every SM) and its
         # backward run beside the GCN's latency-bound first / last kernels (triple index + CSR build, box head) -- as a
         # parallel branch of the captured graph under CUDA-graph replay.
+        # With GT masks (gt_masks) the canvas does not depend on the head: it is issued up front as well, and the head
+        # runs on the main stream for the mask loss only.
+        gt = self._gt_masks(d) if self.gt_masks else None
         main = torch.cuda.current_stream()
         branch = self.branch if self.overlap_canvas else main
         if branch is not main:
             branch.wait_stream(main)
         with torch.cuda.stream(branch):
             layout_vecs = self.layout_embedding(d["objs"])
-            if self.mask_size == 0:
-                canvas = layout_batched(layout_vecs, d["boxes"], d["obj_off"], self.H, self.W,
+            if self.mask_size == 0 or gt is not None:
+                canvas = layout_batched(layout_vecs, d["boxes"], d["obj_off"], self.H, self.W, masks=gt,
                                         max_objs_per_image=d["max_objs"], out_dtype=self.canvas_dtype)
         obj_vecs, boxes_pred = self.model.forward_ragged(d["objs"], res.triplets, res.triplet_type, res.tri_off,
                                                          d["obj_off"])
-        if self.mask_size > 0:
+        mask_loss = None
+        if gt is not None:
+            if self.mask_loss_weight == 0:
+                with torch.no_grad():          # BatchNorm buffers still update; nothing to differentiate
+                    masks_pred = self.model.masks_from_vecs(obj_vecs)
+            else:
+                masks_pred = self.model.masks_from_vecs(obj_vecs)
+                mw = self.mask_loss_weight
+                if self.global_batch is not None:
+                    mw = mw * d["B"] / float(self.global_batch)
+                mask_loss = mask_pred_loss(masks_pred, gt, mw)
+            self.last_masks = masks_pred.detach()
+        elif self.mask_size > 0:
             # predicted masks (meta_models.py:48): the compositor waits for the head; the embedding lookup above stayed
             # on the branch stream
             masks_pred = self.model.masks_from_vecs(obj_vecs)
@@ -247,6 +289,9 @@ class SgToLayoutStep:
         if self.global_batch is not None:
             weight = weight * d["B"] / float(self.global_batch)
         loss, _ = bbox_pred_loss_ragged(boxes_pred, d["boxes"], d["objs"], d["obj_off"], weight)   # pix2pix_model.py:72-85
+        if mask_loss is not None:
+            self.last_mask_loss = mask_loss.detach()
+            loss = loss + mask_loss
         return canvas, loss
 
     def backward(self, d, canvas_grad, prefetch=None):
@@ -282,15 +327,18 @@ class SgToLayoutStep:
     max_graphs = 8
 
     def _graph_key(self, d, G, total):
+        # with GT masks the captured graph reads them from the batch's masks buffer too
+        masks = d.get("masks") if self.gt_masks else None
         return (int(total), int(d["objs"].shape[0]), int(d["B"]), int(d["max_objs"]), d["objs"].data_ptr(),
-                d["boxes"].data_ptr(), d["obj_off"].data_ptr(), G.data_ptr(), tuple(G.shape))
+                d["boxes"].data_ptr(), d["obj_off"].data_ptr(), G.data_ptr(), tuple(G.shape),
+                None if masks is None else (masks.data_ptr(), masks.dtype))
 
     def _capture(self, key, d, G, plan, total):
         dev = self.device
         ent = {"triplets": torch.empty((max(total, 1), 3), dtype=torch.int64, device=dev),
                "types": torch.empty(max(total, 1), dtype=torch.int64, device=dev),
                "tri_off": torch.empty(d["B"] + 1, dtype=torch.int32, device=dev),
-               "keep": (d["objs"], d["boxes"], d["obj_off"], G)}
+               "keep": (d["objs"], d["boxes"], d["obj_off"], G, d.get("masks") if self.gt_masks else None)}
         res = canon_emit(plan, out=(ent["triplets"], ent["types"]))
         ent["tri_off"].copy_(res.tri_off)
         from .canonicalize import CanonResult
@@ -361,6 +409,8 @@ class SgToLayoutStep:
         canonicalization counting pass is enqueued right behind this step's emit pass."""
         if canvas_grad.dtype != self.canvas_dtype:
             raise ValueError("canvas_grad is %s, the canvas is %s" % (canvas_grad.dtype, self.canvas_dtype))
+        if self.gt_masks:
+            self._gt_masks(d)                      # before any work (and outside a graph capture)
         if d.get("_ready") is not None:            # `d` was uploaded on the look-ahead stream
             torch.cuda.current_stream().wait_event(d["_ready"])
         if self.use_graph:

@@ -393,6 +393,15 @@ int csg_adam_multi(int count, void* const* params, const void* const* grads, voi
  * (A > 1) is non-zero.  An image without real objects yields NaN, as the reference's 0 / 0. */
 int csg_box_loss(const float* pred, const float* gt, const long long* objs, int A, const int* obj_off, int B,
                  double weight, float* loss, float* loss_all, float* dpred, csg_stream_t stream);
+/* Mask term of the generator loss (sg2im's compute_generator_loss): loss[0] = weight * F.binary_cross_entropy(pred,
+ * target), the mean over all n elements, and dpred [n] = d loss[0] / d pred, in one pass.  pred fp32 [n]; target [n]
+ * fp32 (target_fmt 0; soft targets in [0, 1]) or int64 (target_fmt 1).  torch's arithmetic: per element
+ * -(t max(log p, -100) + (1 - t) max(log(1 - p), -100)), d/dp = weight (p - t) / max((1 - p) p, 1e-12) / n; a NaN in
+ * pred gives a NaN loss and a NaN in its own dpred element; pred outside [0, 1] is not checked.  n == 0: loss[0] = NaN,
+ * nothing is read.  Deterministic (block partials + one ordered final pass), no host synchronisation. */
+size_t csg_mask_loss_workspace(long long n);
+int csg_mask_loss(const float* pred, const void* target, int target_fmt, long long n, double weight, float* loss,
+                  float* dpred, void* workspace, size_t workspace_bytes, csg_stream_t stream);
 
 /* ---- canonicalization: sg2im/data/base_dataset.py:89-139, scripts/graphs_utils.py:15-155 ------ */
 /* pass 1: per-graph output sizes (cnt0 = type-0 edges, cnt1 = transitive edges; cnt0 = -1 flags a
